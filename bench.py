@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload potts_grid|gauss_chains|hmm64|hmm512|powerlaw|powerlaw_engine|chain1k|chains_engine]
     python bench.py --impl reference ...     # the CPU oracle port of the reference, on the host cores
+    python bench.py ... --dump-outputs DIR   # also write the marginals of the last timed step as DIR/<workload>_marginals.npy
 
 One "step" = one pass of the hot path over one batch of synthetic input:
   potts_grid  (default at every N, BASELINE configs[3]): 50 synchronous sweeps of the 8192^2, K=16 grid, row-sharded over the
@@ -14,7 +15,7 @@ One "step" = one pass of the hot path over one batch of synthetic input:
   powerlaw_engine / chain1k (configs[0]) / chains_engine: the same models through cxb_graph_build + cxb_update_marginals (the
               reference's single entry point; memoised schedules and closed-form plans behind it).
 The default run prints ONE JSON line (rank 0): the potts_grid record, with one sub-record per other config under "others".
-Nothing here reads /root/reference.
+It runs on the tree build() left (the CUDA library and the CPU oracle) and writes nothing there: the tree may be read-only.
 """
 from __future__ import annotations
 
@@ -32,9 +33,27 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # no __pycache__ in the tree
 import __graft_entry__ as entry  # noqa: E402
 
 METRIC, UNIT = "message_updates_per_sec", "updates/s"
+DUMP_BYTES = 60 * 2**20  # --dump-outputs writes at most this much (64 MB in all with the .npy headers)
+
+
+def dump_rows(n_rows, row_bytes):
+    """Indices of the rows of an output that --dump-outputs writes: all of them when they fit DUMP_BYTES, else a fixed, seeded
+    sample (the same for the same arguments, so that two builds can be compared output for output)."""
+    k = max(1, DUMP_BYTES // row_bytes)
+    if n_rows <= k:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(0).choice(n_rows, k, replace=False))
+
+
+def dump_output(args, name, rows):
+    """Write one output of the last timed step (rows chosen by dump_rows) as <DIR>/<workload>_<name>.npy."""
+    out = Path(args.dump_outputs)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / f"{args.workload}_{name}.npy", np.ascontiguousarray(rows))
 
 
 def measured_peaks():
@@ -297,7 +316,6 @@ def run_reference(args):
         return
     import multiprocessing as mp
 
-    subprocess.run(["make", "-C", str(ROOT / "oracle")], check=True, stdout=subprocess.DEVNULL)
     cores = os.cpu_count() or 1
     per_step_budget = max(1.0, min(10.0, 75.0 / max(1, args.steps + args.warmup)))
     _, what = cpu_baseline_workload(args.workload, 0.2)  # the sample's description (and a warm build of the graph code paths)
@@ -396,6 +414,9 @@ def bench_gauss_chains(args, pkg, rank, world, local):
     ms = timed(ch.stream, step, args.steps, 0, world, local, min_ms=args.min_ms)
     steps_timed = timed.last_steps
     launches = pkg.default_api().kernel_launches() - launches0
+    if args.dump_outputs:
+        marg = ch.get_marginals().reshape(T * B, 2)
+        dump_output(args, "marginals", marg[dump_rows(T * B, marg[0].nbytes)])
     # per-launch kernel duration from the library's own CUDA events (same stream)
     for _ in range(min(args.steps, 10)):
         step()
@@ -471,6 +492,10 @@ def bench_potts_grid(args, pkg, rank, world, local):
     launches0 = pkg.default_api().kernel_launches()
     ms = timed(gr.stream, step, args.steps, 0, world, local)
     launches = pkg.default_api().kernel_launches() - launches0
+    if args.dump_outputs:
+        marg = gr.get_marginals().reshape(rows * N, K)
+        dump_output(args, "marginals", marg[dump_rows(rows * N, marg[0].nbytes)])
+        del marg
     kernel_ms = []
     for _ in range(10):
         sweep()
@@ -539,6 +564,8 @@ def bench_hmm64(args, pkg, rank, world, local):
     ms = timed(hm.stream, step, args.steps, 0, world, local, min_ms=args.min_ms)
     steps_timed = timed.last_steps
     launches = pkg.default_api().kernel_launches() - launches0
+    if args.dump_outputs:  # rows = time steps (all chains), fetched one at a time: the full plane does not fit the host
+        dump_output(args, "marginals", np.stack([hm.get_marginals(t, t + 1)[0] for t in dump_rows(T, B * K * 4)]))
     kernel_ms = []
     for _ in range(min(args.steps, 3)):
         step()
@@ -607,6 +634,9 @@ def bench_powerlaw(args, pkg, rank, world, local):
     ms = timed(pw.stream, step, args.steps, 0, world, local, min_ms=args.min_ms)
     steps_timed = timed.last_steps
     launches = pkg.default_api().kernel_launches() - launches0
+    if args.dump_outputs:
+        marg = pw.get_marginals()
+        dump_output(args, "marginals", marg[dump_rows(n, marg[0].nbytes)])
     kernel_ms = []
     for _ in range(10):
         sweep()
@@ -766,6 +796,10 @@ def bench_engine_graph(args, pkg, rank, world, local, which):
     launches0 = api.kernel_launches()
     ms, steps = wall(step, args.steps)
     launches = api.kernel_launches() - launches0
+    if args.dump_outputs:
+        store.check(api.get_values_prepared(store.h, marg_list, ctypes.c_void_p(host_out.data_ptr()), 0))
+        marg = host_out.numpy()
+        dump_output(args, "marginals", marg[dump_rows(n_req, marg[0].nbytes)])
     e2e_ms, e2e_steps = wall(e2e_step, max(2, min(args.steps, 5)))
     clocks = sampler.stop()
     ran = {1: "level schedule", 2: "sequential executor", 3: "memoised level schedule (replay)", 4: "closed-form plan"}.get(
@@ -800,6 +834,7 @@ def run_workload(args, name, pkg, rank, world, local, main_record):
     elif name == "hmm64":
         a.hmm_chains = min(args.hmm_chains, max(1, 1024 // world)) if world > 1 else args.hmm_chains
     if not main_record:
+        a.dump_outputs = None  # only the main record's timed path is dumped
         a.steps, a.warmup = min(args.steps, 3), 3
         if name == "powerlaw_engine":
             a.pl_vars = min(args.pl_vars, 1000000)  # the explicit Signal graph of 10M variables takes minutes to build on the host
@@ -894,7 +929,12 @@ def main():
     ap.add_argument("--pl-sweeps", type=int, default=10)
     ap.add_argument("--engine-chains", type=int, default=4096)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the main record, write the marginals its last step computed as "
+                         "DIR/<workload>_marginals.npy (a fixed, seeded sample of rows when larger than 60 MiB); one GPU only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
@@ -902,8 +942,8 @@ def main():
 
     pkg = entry.load_package()
     rank, world, local = dist_setup(args.gpus)
-    if rank == 0 and not args.no_cpu_baseline:
-        subprocess.run(["make", "-C", str(ROOT / "oracle")], check=True, stdout=subprocess.DEVNULL)
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs runs on one GPU (each rank holds only its shard of the outputs)")
     line = run_workload(args, args.workload, pkg, rank, world, local, main_record=True)
     if NUMA_NOTE:
         line["host_binding"] = dict(NUMA_NOTE)
