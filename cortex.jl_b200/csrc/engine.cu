@@ -35,6 +35,7 @@ constexpr int ERR_NONLISTEN = 512;             // E: non-listening notifications
 constexpr int ERR_FINAL_ORDER = 1024;          // F: final-phase candidates that depend on each other across the per-variable order
 constexpr int ERR_SEQ_OVERFLOW = 2048;         // sequential executor: traversal deeper than the stack (a dependency cycle)
 constexpr int ERR_SEQ_DIVERGED = 4096;         // sequential executor: the reference loop does not terminate on this request
+constexpr int ERR_RULE_SYMBOL = 8192;          // HMM_EMIT: observed symbol out of range (a bad input value, as the oracle reports it)
 constexpr uint32_t PROBE_BIT = 0x80000000u;  // breadth-first list entry: the signal is only probed (see bfs_visit)
 constexpr uint32_t MULTI_BIT = 0x40000000u;  // breadth-first list entry: the reference's depth-first traversal reaches the signal more than once
 constexpr uint32_t ENTRY_ID = 0x3FFFFFFFu;
@@ -743,7 +744,7 @@ __device__ __forceinline__ void rule_cat_warp(const View& e, T* __restrict__ val
     } else if (rule == CXB_RULE_HMM_EMIT) {
         int o = (int)val[(size_t)e.dep_ids[off] * K];
         if (o < 0 || o >= n_sym) {
-            if (lane == 0) atomicOr(e.err_flag, ERR_RULE_ARG);
+            if (lane == 0) atomicOr(e.err_flag, ERR_RULE_SYMBOL);
             o = 0;
         }
 #pragma unroll
@@ -1352,7 +1353,7 @@ __global__ void k_rule_cat(View e, T* __restrict__ val, const uint32_t* list, ui
         for (int c = 0; c < MAXC; ++c) part += acc[c];
         for (int o = G / 2; o > 0; o >>= 1) part += __shfl_xor_sync(gmask, part, o, G);
 #pragma unroll
-        for (int c = 0; c < MAXC; ++c) acc[c] = part + potts_w * acc[c];  // sum_b in[b] + (e^beta - 1) in[a]
+        for (int c = 0; c < MAXC; ++c) acc[c] = (lane + c * G < K) ? part + potts_w * acc[c] : T(0);  // sum_b in[b] + (e^beta - 1) in[a]; padding stays 0
     } else if (rule == CXB_RULE_CAT_TABLE) {
         // stage the incoming message, then every lane contracts its own output components
         T* my_in = sh_in + (size_t)g * K;
@@ -1380,7 +1381,7 @@ __global__ void k_rule_cat(View e, T* __restrict__ val, const uint32_t* list, ui
         if (active && nd > 0) {
             o = (int)val[(size_t)dep_ids[off] * K];
             if (o < 0 || o >= n_sym) {
-                atomicOr(e.err_flag, ERR_RULE_ARG);
+                atomicOr(e.err_flag, ERR_RULE_SYMBOL);
                 o = 0;
             }
         }
@@ -2021,6 +2022,37 @@ struct DeviceEngine {
     int n_keys() const { return (int)key_ftype.size() + 2; }
     int key_no_rule() const { return (int)key_ftype.size() + 1; }
 
+    // launch shape of k_rule_cat for one categorical rule (rule < 0: the family product): G lanes and maxc components per
+    // lane for each signal, CAT_THREADS threads a block, dynamic shared memory (both CAT_TABLE orientations + staged inputs)
+    static constexpr int CAT_THREADS = 256;
+    struct CatShape {
+        int G, maxc;
+        size_t smem;
+    };
+    CatShape cat_shape(int rule) const {
+        CatShape c{1, 0, 0};
+        while (c.G < dim && c.G < 32) c.G <<= 1;
+        c.maxc = (dim + c.G - 1) / c.G;
+        c.smem = ((rule == CXB_RULE_CAT_TABLE ? 2 * (size_t)dim * dim : 0) + (size_t)(CAT_THREADS / c.G) * dim) * esz();
+        return c;
+    }
+    int32_t check_cat_shape(const CatShape& c) {
+        if (c.smem > 200 * 1024 || c.maxc > 16) {
+            err = "categorical value_dim too large for the generic engine (use the structured HMM engine)";
+            return CXB_ERR_BAD_ARG;
+        }
+        return CXB_OK;
+    }
+    // every categorical rule of the engine fits k_rule_cat: checked before a request touches any state, because a width
+    // refused at launch time would leave the levels before it applied (values <= 64 wide never reach the limits)
+    int32_t check_cat_widths() {
+        if (family != CXB_FAMILY_CATEGORICAL) return CXB_OK;
+        int32_t st = check_cat_shape(cat_shape(-1));
+        for (auto it = rules.begin(); !st && it != rules.end(); ++it)
+            if (it->second.kind == CXB_RULE_CAT_TABLE) st = check_cat_shape(cat_shape(CXB_RULE_CAT_TABLE));
+        return st;
+    }
+
     const uint32_t* rule_list_base = nullptr;  // where the members of the level being evaluated live (frontier buffer / a memo's lists)
     FlatDeps rule_flat{nullptr, nullptr, nullptr};  // the memo's flattened dependency lists, indexed like its lists (replay only)
     template <class T>
@@ -2068,16 +2100,10 @@ struct DeviceEngine {
                 } else if (rule == CXB_RULE_POTTS) {
                     w = (T)(std::exp(rd->params.empty() ? 0.0 : rd->params[0]) - 1.0);
                 }
-                int G = 1;
-                while (G < dim && G < 32) G <<= 1;
-                int maxc = (dim + G - 1) / G;
-                const int threads = 256;
-                int gpb = threads / G;
-                size_t smem = ((rule == CXB_RULE_CAT_TABLE ? 2 * (size_t)dim * dim : 0) + (size_t)gpb * dim) * sizeof(T);
-                if (smem > 200 * 1024 || maxc > 16) {
-                    err = "categorical value_dim too large for the generic engine (use the structured HMM engine)";
-                    return CXB_ERR_BAD_ARG;
-                }
+                const CatShape cs = cat_shape(rule);
+                const int G = cs.G, maxc = cs.maxc, gpb = CAT_THREADS / G, threads = CAT_THREADS;
+                const size_t smem = cs.smem;
+                if (int32_t st = check_cat_shape(cs)) return st;
                 unsigned grid = std::min(cdiv(cnt, gpb), 148u * 8u);  // persistent: 8 blocks of 256 threads per SM
                 FlatDeps fd{nullptr, nullptr, nullptr};
                 if (rule_flat.off) fd = FlatDeps{rule_flat.off + off, rule_flat.src, rule_flat.low + off};
@@ -2168,8 +2194,12 @@ struct DeviceEngine {
     int32_t flags_to_status(int f) {
         if (!f) return CXB_OK;
         cudaMemsetAsync(d_flags.p, 0, sizeof(int), stream);
+        if (f & ERR_RULE_SYMBOL) {
+            err = "HMM_EMIT: symbol out of range";
+            return CXB_ERR_BAD_ARG;
+        }
         if (f & ERR_RULE_ARG) {
-            err = "rule kernel rejected its arguments (no dependencies, symbol out of range or unknown rule kind)";
+            err = "rule kernel rejected its arguments (no dependencies or unknown rule kind)";
             return CXB_ERR_NO_RULE;
         }
         if (f & ERR_SEQ_DIVERGED) {
@@ -3007,13 +3037,8 @@ struct DeviceEngine {
             hit = true;
             return CXB_OK;
         }
-        if (m->plan > 0) {
-            if ((st = run_plan(*m))) return st;
-            last_ran = CXB_RAN_PLAN;
-        } else {
-            if ((st = replay_levels(*m))) return st;
-            last_ran = CXB_RAN_REPLAY;
-        }
+        last_ran = m->plan > 0 ? CXB_RAN_PLAN : CXB_RAN_REPLAY;  // also when a rule refuses its arguments, as update_level does
+        if ((st = m->plan > 0 ? run_plan(*m) : replay_levels(*m))) return st;
         if (N) CXB_CUDA(cudaMemcpyAsync(d_props.p, m->post_props.p, N, cudaMemcpyDeviceToDevice, stream));
         if (NC) CXB_CUDA(cudaMemcpyAsync(d_nib.p, m->post_nib.p, NC * sizeof(uint64_t), cudaMemcpyDeviceToDevice, stream));
         if ((st = check_flags())) return st;  // a rule rejected its arguments (the only error a replay can meet)
@@ -3082,6 +3107,7 @@ struct DeviceEngine {
         last_ran = 0;
         int32_t st = ensure_device();
         if (st) return st;
+        if ((st = check_cat_widths())) return st;
         CXB_CUDA(cudaMemsetAsync(d_kind_count.p, 0, 8 * sizeof(unsigned long long), stream));
         if (schedule == CXB_SCHEDULE_SEQUENTIAL || (schedule == CXB_SCHEDULE_AUTO && hand_wired && small_values())) {
             if (!small_values()) {

@@ -98,6 +98,7 @@ enum {
     CXB_RULE_CAT_TABLE = 3,    /* out[x_v] = sum_{x_u} psi[x_lo][x_hi] * in[x_u], normalised; params = psi K*K  */
     CXB_RULE_POTTS = 4,        /* psi[a][b] = exp(beta*[a==b]); params = {beta}                                  */
     CXB_RULE_HMM_EMIT = 5,     /* out = normalise(E[:, o]); o = value[0] of the dependency; params = {M, E K*M}  */
+                               /* (o outside [0, M): CXB_ERR_BAD_ARG)                                           */
     CXB_RULE_GAUSS_MV_OBS = 6, /* N(y, r)            test/inference_engine_tests.jl:425-426 (r = 1.0 there)      */
     CXB_RULE_GAUSS_MV_RW = 7,  /* N(m, v + q)        test/inference_engine_tests.jl:427-428 (q = 1.0 there)      */
     CXB_RULE_BETA_BERNOULLI = 8, /* Beta(1 + r, 2 - r) test/inference_engine_tests.jl:256-258                    */
