@@ -11,8 +11,11 @@
 //                linked m2f(v,f)  = normalise(unary * prod_{g != f} m2v(v,g))
 // Potts table psi[a][b] = exp(beta [a==b])  =>  sum_b psi[a][b] m[b] = sum(m) + (e^beta - 1) m[a].
 //
-// Kernel: fused per-pixel pass, HBM-bound (896 B of algorithmic traffic per interior pixel at K=16 fp32:
-// read 4 m2f + unary, write 4 m2v + 4 m2f + marginal).  LP = K / (16 B / sizeof(T)) lanes cooperate on one
+// Kernel: fused per-pixel pass, HBM-bound (640 B of traffic per interior pixel at K=16 fp32: read 4 m2f + unary, write
+// 4 m2f + marginal).  Every m2v is computed, but only rows 0 and H - 1 store theirs: the others are a function of this
+// sweep's input m2f, which stays intact until the next sweep, so k_potts_m2v rebuilds them bit for bit on the first read
+// of an m2v plane (cxb_grid_get_messages).  No later sweep reads them; storing them would add 256 B per pixel.
+// CXB_GRID_EAGER_M2V=1 stores every m2v every sweep (896 B per pixel).  LP = K / (16 B / sizeof(T)) lanes cooperate on one
 // pixel, each lane moving 16-byte vectors, so a warp touches 32*16 = 512 contiguous bytes per plane per
 // instruction; K-sums are 2-4 warp-shuffle steps.  m2f planes are double buffered (sweep reads `cur`, writes
 // `nxt`), every value is read exactly once.  Row sharding: the up/down messages of the first/last local row
@@ -78,9 +81,33 @@ __device__ __forceinline__ T rcp_pos(T x) {
     }
 }
 
+// loop phase of one factor: m2v(v, f) = normalise(S + w * in), S = sum(in), stored at plane + o when `store`; an absent
+// factor gives the neutral element and stores nothing. The sweep and k_potts_m2v both call this, so a rebuilt m2v is
+// bit-identical to the one the sweep multiplied with. (The store sits inside the branch: computing its address outside it
+// costs the fp32 sweep up to 9 registers.)
+template <class T, int E, int LP>
+__device__ __forceinline__ void potts_m2v(const T (&in)[E], bool ex, T w, T (&mv)[E], bool store, void* plane, size_t o) {
+    const T S = group_sum<T, E, LP>(in);
+#pragma unroll
+    for (int k = 0; k < E; ++k) mv[k] = S + w * in[k];
+    const T tot = group_sum<T, E, LP>(mv);  // every lane shuffles, present factor or not
+    if (ex) {
+        const T inv = rcp_pos<T>(tot);
+#pragma unroll
+        for (int k = 0; k < E; ++k) mv[k] = mv[k] * inv;
+        if (store) store_vec<T, E>((T*)plane + o, mv);
+    } else {
+#pragma unroll
+        for (int k = 0; k < E; ++k) mv[k] = T(1);
+    }
+}
+
 struct GridView {
     long long H, W;
     int has_up, has_down;
+    // 1: store every m2v plane (CXB_GRID_EAGER_M2V=1). 0: store only rows 0 and H - 1, whose up / down inputs may come from
+    // a halo buffer that a neighbour can overwrite before the planes are read; k_potts_m2v rebuilds the other rows on read
+    int eager_m2v;
     const void* unary;       // [H][W][K]
     const void* m2f_cur[4];  // [H][W][K] per direction (message from the pixel towards direction d)
     void* m2f_nxt[4];
@@ -135,23 +162,12 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
             }
         }
     }
-    // loop phase: m2v(v, f_d) = normalise(S + w * in)
+    // loop phase
+    const bool store_mv = valid && (g.eager_m2v || i == 0 || i + 1 == g.H);
     T mv[4][E];
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
-        T S = group_sum<T, E, LP>(in[d]);
-#pragma unroll
-        for (int k = 0; k < E; ++k) mv[d][k] = S + w * in[d][k];
-        T tot = group_sum<T, E, LP>(mv[d]);
-        if (ex[d]) {
-            const T inv = rcp_pos<T>(tot);
-#pragma unroll
-            for (int k = 0; k < E; ++k) mv[d][k] = mv[d][k] * inv;
-            if (valid) store_vec<T, E>((T*)g.m2v[d] + o, mv[d]);
-        } else {
-#pragma unroll
-            for (int k = 0; k < E; ++k) mv[d][k] = T(1);  // absent factor: neutral element of the product
-        }
+        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], store_mv, g.m2v[d], o);
     }
     // final phase: marginal, then the linked m2f (products in ascending factor order, left to right)
     {
@@ -189,6 +205,45 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
         // overlapped with the rest of the sweep; cxb_grid_sweep publishes a sweep counter after the kernel
         if (d == 0 && valid && i == 0 && g.peer_up) store_vec<T, E>((T*)g.peer_up + (size_t)j * K + (size_t)lane * E, acc);
         if (d == 3 && valid && i + 1 == g.H && g.peer_down) store_vec<T, E>((T*)g.peer_down + (size_t)j * K + (size_t)lane * E, acc);
+    }
+}
+
+// The m2v planes of rows 1 .. H - 2, which a sweep with eager_m2v == 0 does not store, rebuilt from the m2f planes that sweep
+// read (g.m2f_cur): they stay intact until the next sweep, whose own m2v supersede these. Rows 1 .. H - 2 take their up and
+// down inputs from this shard's planes, never from a halo buffer. Lane layout as in k_potts_sweep; no store where the factor
+// is absent, so those slots keep the zeros of init.
+template <class T, int K, int E>
+__global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
+    constexpr int LP = K / E;
+    const long long npix = (g.H - 2) * g.W;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    long long q = gid / LP;
+    const int lane = (int)(gid % LP);
+    const bool valid = q < npix;
+    if (!valid) q = npix - 1;  // keep the whole warp in the shuffles
+    const long long pix = q + g.W;
+    const long long j = pix % g.W;
+    const size_t o = (size_t)pix * K + (size_t)lane * E;
+    const bool ex[4] = {true, j > 0, j + 1 < g.W, true};
+    const T* src[4];
+    src[0] = (const T*)g.m2f_cur[3] + o - (size_t)g.W * K;
+    src[1] = (const T*)g.m2f_cur[2] + o - K;
+    src[2] = (const T*)g.m2f_cur[1] + o + K;
+    src[3] = (const T*)g.m2f_cur[0] + o + (size_t)g.W * K;
+    T in[4][E];  // all four loads in flight before the first store
+#pragma unroll
+    for (int d = 0; d < 4; ++d) {
+        if (ex[d]) {
+            load_vec<T, E>(src[d], in[d]);
+        } else {
+#pragma unroll
+            for (int k = 0; k < E; ++k) in[d][k] = T(1);
+        }
+    }
+#pragma unroll
+    for (int d = 0; d < 4; ++d) {
+        T mv[E];
+        potts_m2v<T, E, LP>(in[d], ex[d], w, mv, valid, g.m2v[d], o);
     }
 }
 
@@ -247,6 +302,9 @@ struct Grid {
     unsigned long long job_no = 0;
     unsigned sweep_no = 0;                      // sweeps since the last reset (parity of the halo buffers)
     unsigned long long halo_timeout_ns = 20ull * 1000000000ull;  // CXB_GRID_HALO_TIMEOUT_MS overrides (tests)
+    // m2v planes: a sweep stores only their first and last rows unless eager_m2v (CXB_GRID_EAGER_M2V=1); m2v_pending = the
+    // other rows of the last sweep are not yet rebuilt (flush_m2v)
+    bool eager_m2v = false, m2v_pending = false;
     // after a stream sync: did a halo wait give up on a neighbour?
     int32_t check_halo() {
         if (!peer_halo[0] && !peer_halo[1]) return CXB_OK;
@@ -293,6 +351,7 @@ struct Grid {
         CXB_CUDA(cudaSetDevice(device));
         CXB_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         if (const char* e = getenv("CXB_GRID_HALO_TIMEOUT_MS")) halo_timeout_ns = (unsigned long long)std::max(1, atoi(e)) * 1000000ull;
+        if (const char* e = getenv("CXB_GRID_EAGER_M2V")) eager_m2v = atoi(e) != 0;
         CXB_CUDA(cudaEventCreate(&ev0));
         CXB_CUDA(cudaEventCreate(&ev1));
         CXB_CUDA(unary.reserve(plane()));
@@ -314,6 +373,7 @@ struct Grid {
     }
     int32_t reset() {
         CXB_CUDA(cudaSetDevice(device));
+        if (int32_t st = flush_m2v()) return st;  // before the fill below overwrites the m2f planes it reads
         size_t n = (size_t)4 * H * W * K, nh = (size_t)4 * W * K;
         double u = 1.0 / K;
         for (int b = 0; b < 2; ++b) dtype == CXB_F32 ? fill<float>(m2f[b].p, n, u) : fill<double>(m2f[b].p, n, u);
@@ -330,14 +390,34 @@ struct Grid {
         have_msgs = true;
         return CXB_OK;
     }
+    // the views of both kernels: m2f planes of buffer `in` are read, those of in ^ 1 written
+    GridView view(int in) const {
+        GridView g{};
+        g.H = H;
+        g.W = W;
+        g.has_up = has_up;
+        g.has_down = has_down;
+        g.eager_m2v = eager_m2v;
+        for (int d = 0; d < 4; ++d) {
+            g.m2f_cur[d] = m2f[in].p + (size_t)d * plane();
+            g.m2f_nxt[d] = m2f[in ^ 1].p + (size_t)d * plane();
+            g.m2v[d] = m2v.p + (size_t)d * plane();
+        }
+        return g;
+    }
+    // k_potts_sweep over every pixel, or k_potts_m2v over rows 1 .. H - 2
     template <class T, int E>
-    int32_t launch_k(const GridView& g, T w) {
-        long long threads = H * W * (K / E);
+    int32_t launch_k(const GridView& g, bool m2v_only) {
+        const T w = (T)(std::exp(beta) - 1.0);
+        long long threads = (m2v_only ? H - 2 : H) * W * (K / E);
         unsigned grid = cdiv((size_t)threads, 256);
         switch (K / E) {
 #define CASE(LPV)                                                                                      \
     case LPV:                                                                                          \
-        CXB_LAUNCH((k_potts_sweep<T, LPV * E, E>), grid, 256, 0, stream, g, w);                        \
+        if (m2v_only)                                                                                  \
+            CXB_LAUNCH((k_potts_m2v<T, LPV * E, E>), grid, 256, 0, stream, g, w);                      \
+        else                                                                                           \
+            CXB_LAUNCH((k_potts_sweep<T, LPV * E, E>), grid, 256, 0, stream, g, w);                    \
         break;
             CASE(1)
             CASE(2)
@@ -355,17 +435,8 @@ struct Grid {
             return CXB_ERR_STATE;
         }
         CXB_CUDA(cudaSetDevice(device));
-        GridView g;
-        g.H = H;
-        g.W = W;
-        g.has_up = has_up;
-        g.has_down = has_down;
+        GridView g = view(cur);
         g.unary = cur_unary ? cur_unary : unary.p;
-        for (int d = 0; d < 4; ++d) {
-            g.m2f_cur[d] = m2f[cur].p + (size_t)d * plane();
-            g.m2f_nxt[d] = m2f[cur ^ 1].p + (size_t)d * plane();
-            g.m2v[d] = m2v.p + (size_t)d * plane();
-        }
         g.marg = cur_marg ? cur_marg : marg.p;
         // halo buffers are double buffered by sweep parity: sweep s reads parity s & 1 (written by the neighbours' sweep
         // s - 1, or by the caller's exchange) and pushes its own boundary rows into the neighbours' parity (s + 1) & 1
@@ -374,15 +445,15 @@ struct Grid {
         g.halo_down = halo_recv.p + par + row();
         g.peer_up = peer_halo[0] ? peer_halo[0] + nxt_par + row() : nullptr;   // the upper neighbour's halo_down
         g.peer_down = peer_halo[1] ? peer_halo[1] + nxt_par : nullptr;         // the lower neighbour's halo_up
-        double w = std::exp(beta) - 1.0;
         const bool fused = peer_halo[0] || peer_halo[1];
         if (fused && sweep_no > 0)  // the neighbours have finished sweep sweep_no - 1 (their boundary rows have landed here)
             CXB_LAUNCH(k_halo_wait, 1, 1, 0, stream, peer_halo[0] ? flags.p + 0 : nullptr, peer_halo[1] ? flags.p + 1 : nullptr, sweep_no,
                        halo_timeout_ns, flags.p + 2);
         CXB_CUDA(cudaEventRecord(ev0, stream));
-        int32_t st = dtype == CXB_F32 ? launch_k<float, 4>(g, (float)w) : launch_k<double, 2>(g, w);
+        int32_t st = dtype == CXB_F32 ? launch_k<float, 4>(g, false) : launch_k<double, 2>(g, false);
         if (st) return st;
         CXB_CUDA(cudaEventRecord(ev1, stream));
+        m2v_pending = !eager_m2v;
         if (fused)  // tell the neighbours: my sweep sweep_no is complete (I am their lower / upper neighbour)
             CXB_LAUNCH(k_halo_signal, 1, 1, 0, stream, peer_flags[0] ? peer_flags[0] + 1 : nullptr, peer_flags[1] ? peer_flags[1] + 0 : nullptr,
                        sweep_no + 1);
@@ -396,6 +467,20 @@ struct Grid {
             long long horz = H * (W - 1) * 2;
             *n_updates = 2 * (vert + horz) + H * W;  // m2v + m2f + marginals
         }
+        return CXB_OK;
+    }
+    // rebuild the m2v rows the last sweep did not store, from the m2f planes it read (m2f[cur ^ 1] once it has run); enqueued
+    // on `stream` after the sweep and outside ev0 / ev1
+    int32_t flush_m2v() {
+        if (!m2v_pending) return CXB_OK;
+        CXB_CUDA(cudaSetDevice(device));
+        if (H > 2) {
+            const GridView g = view(cur ^ 1);
+            int32_t st = dtype == CXB_F32 ? launch_k<float, 4>(g, true) : launch_k<double, 2>(g, true);
+            if (st) return st;
+            CXB_CUDA(cudaGetLastError());
+        }
+        m2v_pending = false;
         return CXB_OK;
     }
     // Host entry point of one JOB: evidence from (pinned) host memory, n_sweeps synchronous sweeps, marginals back to host
@@ -588,6 +673,8 @@ int32_t cxb_grid_get_messages(cxb_grid* g, int32_t which, void* out_host) try {
     }
     const unsigned char* src = which < 4 ? h->m2v.p + (size_t)which * h->plane() : h->m2f[h->cur].p + (size_t)(which - 4) * h->plane();
     GR_CUDA(g, cudaSetDevice(h->device));
+    if (which < 4)
+        if (int32_t st = h->flush_m2v()) return st;
     GR_CUDA(g, cudaMemcpyAsync(out_host, src, h->plane(), cudaMemcpyDeviceToHost, h->stream));
     GR_CUDA(g, cudaStreamSynchronize(h->stream));
     return CXB_OK;

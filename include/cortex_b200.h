@@ -368,7 +368,11 @@ int32_t cxb_grid_get_marginals(cxb_grid* g, void* out_host);
  * while this job's sweeps run (two evidence and two marginal buffers). marginals_out_host is complete when cxb_grid_sync
  * returns. Messages carry over from the previous job (call cxb_grid_reset_messages, all shards idle, for a cold start). */
 int32_t cxb_grid_infer_host(cxb_grid* g, const void* unary_host, void* marginals_out_host, int32_t n_sweeps, int64_t* n_updates_out);
-/* message planes for parity: which = 0..3 m2v from the (up,left,right,down) factor, 4..7 m2f to them; D2H */
+/* message planes for parity: which = 0..3 m2v from the (up,left,right,down) factor, 4..7 m2f to them; D2H.
+ * A sweep computes every m2v but stores only those of its first and last rows; the first read of an m2v plane after a
+ * sweep rebuilds the other rows, bit for bit, from the m2f messages that sweep read (one extra kernel on the grid's stream,
+ * about 34 GB of traffic at 8192^2, K = 16 fp32; later reads of the same sweep's planes launch nothing).
+ * CXB_GRID_EAGER_M2V=1 at cxb_grid_create stores every m2v every sweep instead. */
 int32_t cxb_grid_get_messages(cxb_grid* g, int32_t which, void* out_host);
 void* cxb_grid_stream(cxb_grid* g);
 int32_t cxb_grid_last_kernel_ms(cxb_grid* g, float* ms_out);
