@@ -12,7 +12,9 @@
 // For K <= 64 (fp32) the lane's columns of Tbl live in REGISTERS (2 x 64 values), v is staged in a per-warp
 // shared-memory line and read back with broadcast 128-bit loads, so a step is K*K/32 FFMAs + K/4 LDS per warp
 // and no block-level barrier.  Larger K stream Tbl through shared memory in row tiles shared by the 8 chains of
-// the CTA.  (The tcgen05 path for K = 512 named by the north star is future work: see DESIGN.md.)
+// the CTA.
+// Which kernel runs: K = 64 fp32 -> k_hmm64_pass; fp32, K >= 128 a multiple of 64, M <= 64 -> the tcgen05 path of
+// hmm_tc.cuh (k_hmm_tc_step_pair); every other (K, dtype), and CXB_HMM_NO_TC=1 -> k_hmm_pass.
 #include <algorithm>
 #include <cmath>
 #include <type_traits>
@@ -21,7 +23,6 @@
 
 #include "common.cuh"
 #include "hmm_tc.cuh"
-#include "hmm64_tc.cuh"
 
 namespace cxb {
 
@@ -386,356 +387,6 @@ k_hmm64_pass(const float* __restrict__ tbl, const float* __restrict__ emis_n, co
     }
 }
 
-// ---- K = 64, fp32: TWO warps per chain (one CTA of 64 threads per chain: 2,048 warps = 3.5 per scheduler at B = 1,024) ----
-// MEASURED ALTERNATIVE, off by default (see launch_k64): slower than one warp per chain at config-3 size.
-// With one warp per chain the batch of config 3 leaves 1.75 warps per scheduler and every step pays its dependent chain
-// (shared loads -> 64 FFMA2 -> shuffles) almost in full (630 cycles per step against a 221-cycle FMA-pipe floor). Here warp h
-// of a chain owns the output states [32 h, 32 h + 32): lane (cg = lane / 4, rg = lane % 4) holds the 16 x 4 tile
-// tbl[16 rg .. 16 rg + 15][32 h + 4 cg .. + 3] as 32 packed pairs (half the registers), does 32 FFMA2 per step on four
-// 128-bit shared loads, and a 3-shuffle transpose-reduce over the four row groups leaves output state 32 h + lane in the
-// lane (one float per lane: 128 contiguous bytes per warp in every global access). The two warps exchange the carried
-// message, the maximum of their half (exact power-of-two scaling, as above) and the partial sums of the deferred exact
-// normalisation through double-buffered shared memory with ONE 64-thread barrier per step. The exactly normalised
-// message / marginal of step s-5 leaves during step s (per-warp pipelined butterfly, 4 steps; cross-warp total, 1 more).
-template <bool FWD, bool EM_SMEM>
-__global__ void __launch_bounds__(64, 7)  // 7 chains per SM: 1,024 chains in one wave on 148 SMs
-k_hmm64_split(const float* __restrict__ tbl, const float* __restrict__ emis_n, const uint8_t* __restrict__ obs,
-              float* __restrict__ fwd, float* __restrict__ marg, long long B, long long Tn, int n_sym) {
-    constexpr int K = 64, LOOK = 8, LAG = 5, VS = 72;  // VS: states 32 .. 63 are shifted by 4 banks
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float* sh_v = reinterpret_cast<float*>(smem_raw);  // [2][VS] carried message, double buffered
-    float* sh_mx = sh_v + 2 * VS;                      // [2][2] max of each warp's half of the carried message
-    float* sh_tot = sh_mx + 4;                         // [2][2] per-warp sums of the value that leaves next
-    float* sh_em = sh_tot + 4;                         // [M][64] emission messages (if they fit)
-    const int h = threadIdx.x >> 5, lane = threadIdx.x & 31, cg = lane >> 2, rg = lane & 3;
-    const long long b = blockIdx.x;
-    float2 a2[4][8];  // a2[jj][ip] = (tbl[16 rg + 2 ip][j], tbl[16 rg + 2 ip + 1][j]), j = 32 h + 4 cg + jj
-#pragma unroll
-    for (int jj = 0; jj < 4; ++jj)
-#pragma unroll
-        for (int ip = 0; ip < 8; ++ip) {
-            const int j = 32 * h + 4 * cg + jj, i = 16 * rg + 2 * ip;
-            a2[jj][ip] = make_float2(tbl[(size_t)i * K + j], tbl[(size_t)(i + 1) * K + j]);
-        }
-    if (EM_SMEM)
-        for (int x = threadIdx.x; x < n_sym * K; x += blockDim.x) sh_em[x] = emis_n[x];
-    if (threadIdx.x < 4) {
-        sh_mx[threadIdx.x] = 1.0f;
-        sh_tot[threadIdx.x] = 1.0f;
-    }
-    __syncthreads();
-    const int my_state = 32 * h + lane;
-    const int my_slot = my_state + 4 * h;            // where this lane's state lives in sh_v
-    const int rd_off = 16 * rg + 4 * (rg >> 1);      // this lane's 16 input states
-
-    auto time_of = [&](long long step) { return FWD ? step : Tn - 1 - step; };
-    auto load_obs_block = [&](long long step0) -> int {  // lane l fetches the symbol of step0 + l
-        long long st = step0 + lane;
-        return (st < Tn) ? (int)obs[(size_t)time_of(st) * B + b] : 0;
-    };
-    auto fwd_at = [&](long long step) -> float {  // BWD: forward message of `step` for this lane's state
-        return (step < Tn) ? __ldcs(&fwd[((size_t)time_of(step) * B + b) * K + my_state]) : 0.0f;
-    };
-    int obs_cur = 0, obs_next = load_obs_block(0);
-    float a_cur[LOOK], a_nxt[LOOK];
-#pragma unroll
-    for (int u = 0; u < LOOK; ++u) {
-        a_cur[u] = 0.0f;
-        a_nxt[u] = FWD ? 0.0f : fwd_at(u);
-    }
-    float ring[LOOK];  // what steps s-1 .. s-8 leave behind (FWD: the message, BWD: fwd * bwd)
-#pragma unroll
-    for (int u = 0; u < LOOK; ++u) ring[u] = 0.0f;
-    float p1 = 0.0f, p2 = 0.0f, p3 = 0.0f;  // butterfly partial sums in flight (one level per step)
-
-    auto step = [&](auto gen_tag, long long s, int slot, float a_now) {
-        constexpr bool GEN = decltype(gen_tag)::value;
-        const int cur = (int)(s & 1), prv = cur ^ 1;
-        int o = __shfl_sync(0xffffffffu, obs_cur, (int)(s & 31));
-        if (o >= n_sym) o = n_sym - 1;
-        const float em = EM_SMEM ? sh_em[o * K + my_state] : __ldg(emis_n + (size_t)o * K + my_state);
-        // what the two warps left at the previous step: maxima of the carried message, sums of the value of step s-5
-        const float2 mx2 = *reinterpret_cast<const float2*>(sh_mx + 2 * prv);
-        const float2 tt2 = *reinterpret_cast<const float2*>(sh_tot + 2 * prv);
-        const float r = hmm_pow2_inv(fmaxf(mx2.x, mx2.y));
-        if (!GEN || (s >= LAG && s - LAG < Tn)) {
-            const float q = hmm_rcp(tt2.x + tt2.y);
-            float* dst = FWD ? fwd : marg;
-            __stcs(&dst[((size_t)time_of(s - LAG) * B + b) * K + my_state], ring[(slot + LOOK - LAG) % LOOK] * q);
-        }
-        float tot;
-        {   // pipelined butterfly over the warp's 32 states: step s-1 enters, step s-4 completes
-            const float x1 = ring[(slot + LOOK - 1) % LOOK];
-            const float n1 = x1 + __shfl_xor_sync(0xffffffffu, x1, 16);
-            const float n2 = p1 + __shfl_xor_sync(0xffffffffu, p1, 8);
-            const float n3 = p2 + __shfl_xor_sync(0xffffffffu, p2, 4);
-            const float m4 = p3 + __shfl_xor_sync(0xffffffffu, p3, 2);
-            tot = m4 + __shfl_xor_sync(0xffffffffu, m4, 1);
-            p1 = n1;
-            p2 = n2;
-            p3 = n3;
-        }
-        float unew = 0.0f;
-        if (!GEN || s < Tn) {
-            float val = 1.0f;
-            if (!GEN || s > 0) {
-                const float4* vp = reinterpret_cast<const float4*>(sh_v + cur * VS + rd_off);
-                float4 v4[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v4[q] = vp[q];
-                float2 c[4], e[4];  // 8 independent FFMA2 chains of length 4
-#pragma unroll
-                for (int jj = 0; jj < 4; ++jj) c[jj] = e[jj] = make_float2(0.0f, 0.0f);
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float2 lo = make_float2(v4[q].x, v4[q].y), hi = make_float2(v4[q].z, v4[q].w);
-#pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) c[jj] = ffma2(a2[jj][2 * q], lo, c[jj]);
-#pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) e[jj] = ffma2(a2[jj][2 * q + 1], hi, e[jj]);
-                }
-                float acc[4];
-#pragma unroll
-                for (int jj = 0; jj < 4; ++jj) acc[jj] = (c[jj].x + e[jj].x) + (c[jj].y + e[jj].y);
-                // transpose-reduce over the four row groups: lane rg ends with column jj = rg of its column group
-                const bool b0 = rg & 1, b1 = rg & 2;
-                const float kA = (b0 ? acc[1] : acc[0]) + __shfl_xor_sync(0xffffffffu, b0 ? acc[0] : acc[1], 1);
-                const float kB = (b0 ? acc[3] : acc[2]) + __shfl_xor_sync(0xffffffffu, b0 ? acc[2] : acc[3], 1);
-                val = (b1 ? kB : kA) + __shfl_xor_sync(0xffffffffu, b1 ? kA : kB, 2);
-            }
-            unew = (!GEN || s > 0) ? em * val * r : em;
-            ring[slot] = FWD ? unew : a_now * val;
-            sh_v[prv * VS + my_slot] = unew;
-        }
-        float mx;
-        asm("redux.sync.max.f32 %0, %1, 0xffffffff;" : "=f"(mx) : "f"(unew));
-        if (lane == 0) {
-            sh_mx[2 * cur + h] = mx;
-            sh_tot[2 * cur + h] = tot;
-        }
-        __syncthreads();  // the chain's two warps: message, maxima and sums of this step are visible
-    };
-
-    for (long long s0 = 0; s0 < Tn + LAG; s0 += LOOK) {
-        if ((s0 & 31) == 0) {
-            obs_cur = obs_next;
-            obs_next = load_obs_block(s0 + 32);
-        }
-        if (!FWD) {
-#pragma unroll
-            for (int u = 0; u < LOOK; ++u) {
-                a_cur[u] = a_nxt[u];
-                a_nxt[u] = fwd_at(s0 + LOOK + u);
-            }
-            if (s0 + 32 < Tn && lane < 2)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(&fwd[((size_t)time_of(s0 + 32) * B + b) * K + 32 * lane]));
-        }
-        if (s0 >= LOOK && s0 + LOOK <= Tn) {
-#pragma unroll
-            for (int uu = 0; uu < LOOK; ++uu) step(std::false_type{}, s0 + uu, uu, a_cur[uu]);
-        } else {
-#pragma unroll
-            for (int uu = 0; uu < LOOK; ++uu) step(std::true_type{}, s0 + uu, uu, a_cur[uu]);
-        }
-    }
-}
-
-// ---- K = 64, fp32, tensor cores: one CTA of 4 warps per 8 chains (1,024 chains = 128 CTAs, one per SM) -----------------------
-// The sequential recursion leaves one 64 x 64 x 8 product per SM and step: warp w computes output states 16 w .. 16 w + 15 of
-// 8 chains with mma.sync.m16n8k16 (bf16 split operands, hi*hi + hi*lo + lo*hi, fp32 accumulate: 12 MMAs per warp and step
-// instead of 64 FFMA2 per lane), the table fragments stay in registers, the 8 carried messages are exchanged between the
-// 4 warps through a double-buffered bf16 hi/lo image in shared memory (one block barrier per step). Scaling and deferred
-// exact normalisation as in k_hmm64_pass: per-chain max / sum partials travel with the message, the previous step's result
-// is written out, exactly normalised, one step late.
-__device__ __forceinline__ void mma_bf16_m16n8k16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void split_bf16(float x, uint16_t& hi, uint16_t& lo) {
-    const __nv_bfloat16 h = __float2bfloat16_rn(x);
-    hi = __bfloat16_as_ushort(h);
-    lo = __bfloat16_as_ushort(__float2bfloat16_rn(x - __bfloat162float(h)));
-}
-template <bool FWD>
-__global__ void __launch_bounds__(128, 1)
-k_hmm64_mma(const float* __restrict__ tbl, const float* __restrict__ emis_n, const uint8_t* __restrict__ obs,
-            float* __restrict__ fwd, float* __restrict__ marg, long long B, long long Tn, int n_sym) {
-    constexpr int K = 64, NB = 8, VS = 72;  // VS: bf16 elements per chain row (64 + 8: rows start 4 banks apart)
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    uint16_t* sV = reinterpret_cast<uint16_t*>(smem_raw);                  // [2 buffers][2 (hi, lo)][NB][VS]
-    float* sPart = reinterpret_cast<float*>(sV + 2 * 2 * NB * VS);         // [2 buffers][2 (max, sum)][NB][4 warps]
-    uint8_t* sObs = reinterpret_cast<uint8_t*>(sPart + 2 * 2 * NB * 4);    // [2 buffers][32 steps][NB]
-    float* sEm = reinterpret_cast<float*>(sObs + 2 * 32 * NB);             // [n_sym][64]
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-    const int j0 = 16 * warp;
-    const long long b0 = (long long)blockIdx.x * NB;
-    auto time_of = [&](long long step) { return FWD ? step : Tn - 1 - step; };
-
-    // table fragments: M[j][i] = tbl[i][j] (out[j] = sum_i tbl[i][j] v[i]), rows j0 + g / j0 + g + 8, 4 K-steps of 16
-    uint32_t ahi[4][4], alo[4][4];
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks)
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int j = j0 + g + 8 * (r & 1), i = 16 * ks + 2 * t + 8 * (r >> 1);
-            uint16_t h0, l0, h1, l1;
-            split_bf16(tbl[(size_t)i * K + j], h0, l0);
-            split_bf16(tbl[(size_t)(i + 1) * K + j], h1, l1);
-            ahi[ks][r] = (uint32_t)h0 | ((uint32_t)h1 << 16);
-            alo[ks][r] = (uint32_t)l0 | ((uint32_t)l1 << 16);
-        }
-    for (int x = threadIdx.x; x < n_sym * K; x += blockDim.x) sEm[x] = emis_n[x];
-    auto load_obs_block = [&](long long step0, int buf) {  // 32 steps x 8 chains, two entries per thread
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int idx = threadIdx.x * 2 + e, st = idx / NB, n = idx % NB;
-            const long long step = step0 + st;
-            uint8_t o = 0;
-            if (step < Tn && b0 + n < B) o = obs[(size_t)time_of(step) * B + b0 + n];
-            sObs[(buf * 32 + st) * NB + n] = o;
-        }
-    };
-    load_obs_block(0, 0);
-    // this thread's four cells: (state j0 + g + 8 h, chain 2 t + c), h, c in {0, 1}; cell index = 2 h + c (the D fragment order)
-    auto cell_ptr = [&](float* plane, long long step, int h, int c) -> float* {
-        return plane + ((size_t)time_of(step) * B + (size_t)(b0 + 2 * t + c)) * K + j0 + g + 8 * h;
-    };
-    const bool live_c[2] = {b0 + 2 * t < B, b0 + 2 * t + 1 < B};
-    float a_cur[4] = {0, 0, 0, 0}, a_n1[4] = {0, 0, 0, 0}, a_n2[4] = {0, 0, 0, 0};  // BWD: forward message cells of steps s, s+1, s+2
-    auto load_fwd_cells = [&](long long step, float (&dst)[4]) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h)
-#pragma unroll
-            for (int c = 0; c < 2; ++c)
-                dst[2 * h + c] = (step < Tn && live_c[c]) ? __ldcs(cell_ptr(fwd, step, h, c)) : 0.0f;
-    };
-    if (!FWD) {
-        load_fwd_cells(0, a_cur);
-        load_fwd_cells(1, a_n1);
-    }
-    float uprev[4] = {0, 0, 0, 0}, gprev[4] = {0, 0, 0, 0};
-    __syncthreads();
-
-    for (long long s = 0; s <= Tn; ++s) {
-        if ((s & 31) == 0) load_obs_block(s + 32, (int)(((s >> 5) + 1) & 1));  // read 32 steps from now
-        if (!FWD) {
-            load_fwd_cells(s + 2, a_n2);
-            if (s + 16 < Tn && threadIdx.x < 2 * NB)  // pull the forward messages of step s + 16 into L2 (8 chains x 256 B)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(fwd + ((size_t)time_of(s + 16) * B + (size_t)(b0 + (threadIdx.x >> 1))) * K +
-                                                                32 * (threadIdx.x & 1)));
-        }
-        float r[2] = {1.0f, 1.0f};
-        if (s >= 1) {  // totals of step s - 1 (partials of the 4 warps), its exactly normalised write-out, this step's scale
-            const int pb = (int)((s - 1) & 1);
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {
-                const int n = 2 * t + c;
-                const float4 pm = *reinterpret_cast<const float4*>(sPart + ((pb * 2 + 0) * NB + n) * 4);
-                const float4 ps = *reinterpret_cast<const float4*>(sPart + ((pb * 2 + 1) * NB + n) * 4);
-                r[c] = hmm_pow2_inv(fmaxf(fmaxf(pm.x, pm.y), fmaxf(pm.z, pm.w)));
-                const float q = hmm_rcp((ps.x + ps.y) + (ps.z + ps.w));
-                if (live_c[c]) {
-#pragma unroll
-                    for (int h = 0; h < 2; ++h)
-                        __stcs(cell_ptr(FWD ? fwd : marg, s - 1, h, c), (FWD ? uprev[2 * h + c] : gprev[2 * h + c]) * q);
-                }
-            }
-        }
-        if (s < Tn) {
-            float pred[4] = {1.0f, 1.0f, 1.0f, 1.0f};
-            if (s > 0) {
-                const uint16_t* vhi = sV + ((size_t)((s & 1) * 2 + 0) * NB + g) * VS;
-                const uint16_t* vlo = sV + ((size_t)((s & 1) * 2 + 1) * NB + g) * VS;
-                // twelve INDEPENDENT accumulators: the MMAs of a step do not wait for one another (mma.sync latency, not
-                // throughput, is what a step pays for), the partial products are added afterwards
-                float d[4][3][4];
-                uint32_t bh0[4], bh1[4], bl0[4], bl1[4];
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-                    bh0[ks] = *reinterpret_cast<const uint32_t*>(vhi + 16 * ks + 2 * t);
-                    bh1[ks] = *reinterpret_cast<const uint32_t*>(vhi + 16 * ks + 2 * t + 8);
-                    bl0[ks] = *reinterpret_cast<const uint32_t*>(vlo + 16 * ks + 2 * t);
-                    bl1[ks] = *reinterpret_cast<const uint32_t*>(vlo + 16 * ks + 2 * t + 8);
-                }
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-                    for (int p = 0; p < 3; ++p)
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) d[ks][p][i] = 0.0f;
-                    mma_bf16_m16n8k16(d[ks][0], ahi[ks], bh0[ks], bh1[ks]);
-                    mma_bf16_m16n8k16(d[ks][1], ahi[ks], bl0[ks], bl1[ks]);
-                    mma_bf16_m16n8k16(d[ks][2], alo[ks], bh0[ks], bh1[ks]);
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float hh = (d[0][0][i] + d[1][0][i]) + (d[2][0][i] + d[3][0][i]);
-                    const float cr = ((d[0][1][i] + d[0][2][i]) + (d[1][1][i] + d[1][2][i])) + ((d[2][1][i] + d[2][2][i]) + (d[3][1][i] + d[3][2][i]));
-                    pred[i] = hh + cr;
-                }
-            }
-            const uint8_t* ob = sObs + ((size_t)((s >> 5) & 1) * 32 + (s & 31)) * NB;
-            float unew[4], gnew[4];
-            float mx[2] = {0.0f, 0.0f}, sm[2] = {0.0f, 0.0f};
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {
-                int o = ob[2 * t + c];
-                if (o >= n_sym) o = n_sym - 1;
-#pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    const float em = sEm[o * K + j0 + g + 8 * h];
-                    const int cell = 2 * h + c;
-                    unew[cell] = (s > 0) ? em * pred[cell] * r[c] : em;
-                    gnew[cell] = FWD ? unew[cell] : a_cur[cell] * pred[cell];
-                    mx[c] = fmaxf(mx[c], unew[cell]);
-                    sm[c] += gnew[cell];
-                }
-            }
-            // per-chain max / sum over this warp's 16 states: lanes with the same t (xor 4, 8, 16)
-#pragma unroll
-            for (int d = 4; d < 32; d <<= 1)
-#pragma unroll
-                for (int c = 0; c < 2; ++c) {
-                    mx[c] = fmaxf(mx[c], __shfl_xor_sync(0xffffffffu, mx[c], d));
-                    sm[c] += __shfl_xor_sync(0xffffffffu, sm[c], d);
-                }
-            const int wb = (int)(s & 1);
-            if (g == 0) {
-#pragma unroll
-                for (int c = 0; c < 2; ++c) {
-                    sPart[((wb * 2 + 0) * NB + 2 * t + c) * 4 + warp] = mx[c];
-                    sPart[((wb * 2 + 1) * NB + 2 * t + c) * 4 + warp] = sm[c];
-                }
-            }
-            // the carried message of the next step, as bf16 hi / lo rows per chain
-            const int nb = (int)((s + 1) & 1);
-#pragma unroll
-            for (int c = 0; c < 2; ++c)
-#pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    uint16_t hi, lo;
-                    split_bf16(unew[2 * h + c], hi, lo);
-                    sV[((size_t)(nb * 2 + 0) * NB + 2 * t + c) * VS + j0 + g + 8 * h] = hi;
-                    sV[((size_t)(nb * 2 + 1) * NB + 2 * t + c) * VS + j0 + g + 8 * h] = lo;
-                }
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                uprev[i] = unew[i];
-                gprev[i] = gnew[i];
-            }
-        }
-        if (!FWD) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                a_cur[i] = a_n1[i];
-                a_n1[i] = a_n2[i];
-            }
-        }
-        __syncthreads();
-    }
-}
-
 struct Hmm {
     int device = 0, dtype = CXB_F32, K = 0, M = 0;
     long long B = 0, T = 0;
@@ -745,12 +396,10 @@ struct Hmm {
     DBuf<unsigned char> A, At, En, fwd, marg;
     DBuf<uint8_t> obs;
     // tensor-core path (hmm_tc.cuh): table images (forward: rows of A^T, backward: rows of A), message operands, row sums
-    DBuf<uint16_t> tc_img_f, tc_img_b, tc_op[2], tc_op_b[2];  // _b: the backward pass's own ping-pong (paired launches)
+    DBuf<uint16_t> tc_img_f, tc_img_b, tc_op[2], tc_op_b[2];  // _b: the backward pass's own ping-pong
     DBuf<float> tc_part[2], tc_part_b[2];
     bool tc_ready = false;
-    bool tc_paired = true;
     int tc_nt = 64;  // output states per CTA of the tensor-core step kernel (32 or 64)
-    int tc_np = 3;   // bf16 pieces per operand (3: fp32-level accuracy, the default; 2: ~2^-17 per term, CXB_HMM_TC_PIECES=2)
     bool tc_eligible() const {
         if (const char* e = getenv("CXB_HMM_NO_TC"))
             if (atoi(e)) return false;
@@ -816,34 +465,27 @@ struct Hmm {
             // slices of 32 output states when 64-state slices would leave most SMs idle
             int n_sm = 148;
             cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
-            tc_paired = true;  // both passes in one launch per step (k_hmm_tc_step_pair); CXB_HMM_TC_PAIRED=0: one pass after the other
-            if (const char* e = getenv("CXB_HMM_TC_PAIRED")) tc_paired = atoi(e) != 0;
-            // the widest grid that is still resident at once: (chain tiles) x (K / NT slices) x (passes per launch) CTAs, one per SM
-            tc_nt = (tc_bpad() / tc::M_TILE) * (K / 32) * (tc_paired ? 2 : 1) <= n_sm ? 32 : 64;
-            if (const char* e = getenv("CXB_HMM_TC_NT")) tc_nt = atoi(e) == 32 ? 32 : 64;
-            tc_np = 3;
-            if (const char* e = getenv("CXB_HMM_TC_PIECES")) tc_np = atoi(e) == 2 ? 2 : 3;
+            // the widest grid that is still resident at once: (chain tiles) x (K / NT slices) x (2 passes) CTAs, one per SM
+            tc_nt = (tc_bpad() / tc::M_TILE) * (K / 32) * 2 <= n_sm ? 32 : 64;
             std::vector<uint16_t> img;
-            tc::build_table_image((const float*)at.data(), K, tc_nt, tc_np, img);  // forward: pred[j] = sum_i msg[i] A[i][j] -> rows of A^T
+            tc::build_table_image((const float*)at.data(), K, tc_nt, img);  // forward: pred[j] = sum_i msg[i] A[i][j] -> rows of A^T
             CXB_CUDA(tc_img_f.reserve(img.size()));
             CXB_CUDA(cudaMemcpyAsync(tc_img_f.p, img.data(), img.size() * 2, cudaMemcpyHostToDevice, stream));
             CXB_CUDA(cudaStreamSynchronize(stream));
-            tc::build_table_image((const float*)a.data(), K, tc_nt, tc_np, img);   // backward: pred[j] = sum_i A[j][i] msg[i] -> rows of A
+            tc::build_table_image((const float*)a.data(), K, tc_nt, img);   // backward: pred[j] = sum_i A[j][i] msg[i] -> rows of A
             CXB_CUDA(tc_img_b.reserve(img.size()));
             CXB_CUDA(cudaMemcpyAsync(tc_img_b.p, img.data(), img.size() * 2, cudaMemcpyHostToDevice, stream));
             const long long bpad = tc_bpad();
-            const size_t op_elems = (size_t)(bpad / tc::M_TILE) * tc_np * (K / tc::K_CHUNK) * (tc::A_CHUNK_BYTES / 2);
+            const size_t op_elems = (size_t)(bpad / tc::M_TILE) * tc::NP * (K / tc::K_CHUNK) * (tc::A_CHUNK_BYTES / 2);
             for (int i = 0; i < 2; ++i) {
                 CXB_CUDA(tc_op[i].reserve(op_elems));
                 CXB_CUDA(tc_part[i].reserve((size_t)2 * (K / tc_nt) * bpad));
                 CXB_CUDA(cudaMemsetAsync(tc_op[i].p, 0, op_elems * 2, stream));
                 CXB_CUDA(cudaMemsetAsync(tc_part[i].p, 0, (size_t)2 * (K / tc_nt) * bpad * sizeof(float), stream));
-                if (tc_paired) {
-                    CXB_CUDA(tc_op_b[i].reserve(op_elems));
-                    CXB_CUDA(tc_part_b[i].reserve((size_t)2 * (K / tc_nt) * bpad));
-                    CXB_CUDA(cudaMemsetAsync(tc_op_b[i].p, 0, op_elems * 2, stream));
-                    CXB_CUDA(cudaMemsetAsync(tc_part_b[i].p, 0, (size_t)2 * (K / tc_nt) * bpad * sizeof(float), stream));
-                }
+                CXB_CUDA(tc_op_b[i].reserve(op_elems));
+                CXB_CUDA(tc_part_b[i].reserve((size_t)2 * (K / tc_nt) * bpad));
+                CXB_CUDA(cudaMemsetAsync(tc_op_b[i].p, 0, op_elems * 2, stream));
+                CXB_CUDA(cudaMemsetAsync(tc_part_b[i].p, 0, (size_t)2 * (K / tc_nt) * bpad * sizeof(float), stream));
             }
             tc_ready = true;
         }
@@ -864,54 +506,16 @@ struct Hmm {
                    (T*)fwd.p, (T*)marg.p, B, this->T, K, M, tile_rows);
         return CXB_OK;
     }
-    // one launch per time step and pass (hmm_tc.cuh); 2 T + 4 launches
-    int32_t launch_tc() {
-        if (tc_paired) {
-            if (tc_np == 2) return tc_nt == 32 ? launch_tc_pair_nt<32, 2>() : launch_tc_pair_nt<64, 2>();
-            return tc_nt == 32 ? launch_tc_pair_nt<32, 3>() : launch_tc_pair_nt<64, 3>();
-        }
-        if (tc_np == 2) return tc_nt == 32 ? launch_tc_nt<32, 2>() : launch_tc_nt<64, 2>();
-        return tc_nt == 32 ? launch_tc_nt<32, 3>() : launch_tc_nt<64, 3>();
-    }
-    // Paired schedule: launch s runs step s of BOTH passes (forward at time s, backward at time T-1-s): T + 5 launches.
-    // The backward half writes the marginal directly once the forward message of its time step is final (normalised in
-    // place by forward launch t+1, i.e. for T-1-s <= s-2); before that it stores the normalised backward prediction and
-    // k_hmm_tc_combine multiplies the forward messages in at the end (times >= T - s_direct).
-    template <int NT, int NP>
+    int32_t launch_tc() { return tc_nt == 32 ? launch_tc_pair_nt<32>() : launch_tc_pair_nt<64>(); }
+    // One launch per time step (hmm_tc.cuh): launch s runs step s of BOTH passes (forward at time s, backward at time
+    // T-1-s): T + 4 launches. The backward half writes the marginal directly once the forward message of its time step is
+    // final (normalised in place by forward launch t+1, i.e. for T-1-s <= s-2); before that it stores the normalised
+    // backward prediction and k_hmm_tc_combine multiplies the forward messages in at the end (times >= T - s_direct).
+    template <int NT>
     int32_t launch_tc_pair_nt() {
         const int bpad = (int)tc_bpad(), tiles = bpad / tc::M_TILE, n_slices = K / NT;
-        const size_t smem = tc::step_smem_bytes<NT, NP>(M), row = (size_t)B * K;
-        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step_pair<NT, NP, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step_pair<NT, NP, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step_pair<NT, NP, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        // clusters of 4 or 8 slices of a chain tile with a multicast message operand (CXB_HMM_TC_CLUSTER=4|8), when the slices
-        // divide and every cluster of the grid is resident at once (a B200 holds 15 clusters of 8 CTAs of this size: config 3
-        // needs 16, so it falls back)
-        int cl = 1;
-        if (const char* e = getenv("CXB_HMM_TC_CLUSTER")) cl = atoi(e) == 8 ? 8 : atoi(e) == 4 ? 4 : 1;
-        if (cl > 1 && n_slices % cl) cl = 1;
-        if (cl > 1) {
-            cudaLaunchConfig_t q{};
-            q.gridDim = dim3(tiles, n_slices, 2);
-            q.blockDim = dim3(tc::THREADS);
-            q.dynamicSmemBytes = smem;
-            cudaLaunchAttribute qa[1];
-            qa[0].id = cudaLaunchAttributeClusterDimension;
-            qa[0].val.clusterDim.x = 1;
-            qa[0].val.clusterDim.y = cl;
-            qa[0].val.clusterDim.z = 1;
-            q.attrs = qa;
-            q.numAttrs = 1;
-            int n_clusters = 0;
-            const int needed = tiles * (n_slices / cl) * 2, asked = cl;
-            const cudaError_t qe = cl == 8 ? cudaOccupancyMaxActiveClusters(&n_clusters, tc::k_hmm_tc_step_pair<NT, NP, 8>, &q)
-                                           : cudaOccupancyMaxActiveClusters(&n_clusters, tc::k_hmm_tc_step_pair<NT, NP, 4>, &q);
-            if (qe != cudaSuccess || n_clusters < needed) cl = 1;
-            cudaGetLastError();
-            if (getenv("CXB_HMM_TC_VERBOSE"))
-                fprintf(stderr, "cxb_hmm tc: clusters of %d requested: %d resident at once (%s), %d needed -> cluster size %d\n", asked, n_clusters,
-                        cudaGetErrorString(qe), needed, cl);
-        }
+        const size_t smem = tc::step_smem_bytes<NT>(M), row = (size_t)B * K;
+        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step_pair<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         float *fw = (float*)fwd.p, *mg = (float*)marg.p;
         tc::StepArgs2 p{};
         for (int z = 0; z < 2; ++z) {
@@ -924,7 +528,6 @@ struct Hmm {
         p.d[0].tbl_img = (const __nv_bfloat16*)tc_img_f.p;
         p.d[1].tbl_img = (const __nv_bfloat16*)tc_img_b.p;
         const dim3 grid(tiles, n_slices, 2), igrid(bpad / 128, n_slices);
-        const bool pdl = !(getenv("CXB_HMM_TC_NO_PDL") && atoi(getenv("CXB_HMM_TC_NO_PDL")));
         const long long Tn = this->T, s_direct = (Tn + 2) / 2;  // first launch whose backward half sees a final forward message
         DBuf<long long> trace;
         const bool tracing = getenv("CXB_HMM_TC_TRACE") && atoi(getenv("CXB_HMM_TC_TRACE"));
@@ -955,29 +558,20 @@ struct Hmm {
             b.raw_prev = s ? mg + (size_t)(tb + 1) * row : nullptr;
             b.fwd_t = s >= s_direct ? fw + (size_t)tb * row : nullptr;
             if (s == 0) {
-                CXB_LAUNCH((tc::k_hmm_tc_init<true, NT, NP>), igrid, 128, 0, stream, f);
-                CXB_LAUNCH((tc::k_hmm_tc_init<false, NT, NP>), igrid, 128, 0, stream, b);
+                CXB_LAUNCH((tc::k_hmm_tc_init<true, NT>), igrid, 128, 0, stream, f);
+                CXB_LAUNCH((tc::k_hmm_tc_init<false, NT>), igrid, 128, 0, stream, b);
             } else {
                 cudaLaunchConfig_t cfg{};
                 cfg.gridDim = grid;
                 cfg.blockDim = dim3(tc::THREADS);
                 cfg.dynamicSmemBytes = smem;
                 cfg.stream = stream;
-                cudaLaunchAttribute attr[2];
+                cudaLaunchAttribute attr[1];
                 attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                attr[0].val.programmaticStreamSerializationAllowed = (pdl && s > 1) ? 1 : 0;  // launch 1 follows the two init kernels
-                attr[1].id = cudaLaunchAttributeClusterDimension;
-                attr[1].val.clusterDim.x = 1;
-                attr[1].val.clusterDim.y = cl;
-                attr[1].val.clusterDim.z = 1;
+                attr[0].val.programmaticStreamSerializationAllowed = s > 1 ? 1 : 0;  // launch 1 follows the two init kernels
                 cfg.attrs = attr;
-                cfg.numAttrs = cl > 1 ? 2 : 1;
-                if (cl == 8)
-                    CXB_CUDA(cudaLaunchKernelEx(&cfg, tc::k_hmm_tc_step_pair<NT, NP, 8>, p));
-                else if (cl == 4)
-                    CXB_CUDA(cudaLaunchKernelEx(&cfg, tc::k_hmm_tc_step_pair<NT, NP, 4>, p));
-                else
-                    CXB_CUDA(cudaLaunchKernelEx(&cfg, tc::k_hmm_tc_step_pair<NT, NP, 1>, p));
+                cfg.numAttrs = 1;
+                CXB_CUDA(cudaLaunchKernelEx(&cfg, tc::k_hmm_tc_step_pair<NT>, p));
                 ++::cxb::g_kernel_launches;
             }
         }
@@ -1004,143 +598,12 @@ struct Hmm {
         }
         return CXB_OK;
     }
-    template <int NT, int NP>
-    int32_t launch_tc_nt() {
-        const int bpad = (int)tc_bpad(), tiles = bpad / tc::M_TILE, n_slices = K / NT;
-        const size_t smem = tc::step_smem_bytes<NT, NP>(M), row = (size_t)B * K;
-        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step<true, NT, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CXB_CUDA(cudaFuncSetAttribute(tc::k_hmm_tc_step<false, NT, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        float *fw = (float*)fwd.p, *mg = (float*)marg.p;
-        tc::StepArgs a{};
-        a.emis_n = (const float*)En.p;
-        a.B = (int)B;
-        a.Bpad = bpad;
-        a.K = K;
-        a.n_sym = M;
-        const dim3 grid(tiles, n_slices), igrid(bpad / 128, n_slices);
-        DBuf<long long> trace;
-        const bool tracing = getenv("CXB_HMM_TC_TRACE") && atoi(getenv("CXB_HMM_TC_TRACE"));
-        const bool pdl = !(getenv("CXB_HMM_TC_NO_PDL") && atoi(getenv("CXB_HMM_TC_NO_PDL")));
-        if (tracing) {
-            CXB_CUDA(trace.reserve((size_t)tiles * n_slices * 16));
-            CXB_CUDA(cudaMemsetAsync(trace.p, 0, (size_t)tiles * n_slices * 16 * sizeof(long long), stream));
-            a.trace = trace.p;
-        }
-        for (int pass = 0; pass < 2; ++pass) {
-            const bool f = pass == 0;
-            a.tbl_img = (const __nv_bfloat16*)(f ? tc_img_f.p : tc_img_b.p);
-            float* out = f ? fw : mg;
-            for (long long s = 0; s < this->T; ++s) {
-                const long long t = f ? s : this->T - 1 - s, tp = f ? t - 1 : t + 1;
-                a.op_in = (const __nv_bfloat16*)tc_op[(s + 1) & 1].p;
-                a.op_out = (__nv_bfloat16*)tc_op[s & 1].p;
-                a.part_in = tc_part[(s + 1) & 1].p;
-                a.part_out = tc_part[s & 1].p;
-                a.obs_t = obs.p + (size_t)t * B;
-                a.raw_out = out + (size_t)t * row;
-                a.raw_prev = s ? out + (size_t)tp * row : nullptr;
-                a.fwd_t = f ? nullptr : fw + (size_t)t * row;
-                if (s == 0) {
-                    if (f)
-                        CXB_LAUNCH((tc::k_hmm_tc_init<true, NT, NP>), igrid, 128, 0, stream, a);
-                    else
-                        CXB_LAUNCH((tc::k_hmm_tc_init<false, NT, NP>), igrid, 128, 0, stream, a);
-                } else {
-                    cudaLaunchConfig_t cfg{};
-                    cfg.gridDim = grid;
-                    cfg.blockDim = dim3(tc::THREADS);
-                    cfg.dynamicSmemBytes = smem;
-                    cfg.stream = stream;
-                    cudaLaunchAttribute attr[1];
-                    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
-                    cfg.attrs = attr;
-                    cfg.numAttrs = 1;
-                    CXB_CUDA(cudaLaunchKernelEx(&cfg, f ? tc::k_hmm_tc_step<true, NT, NP> : tc::k_hmm_tc_step<false, NT, NP>, a));
-                    ++::cxb::g_kernel_launches;
-                }
-            }
-            const long long t_last = f ? this->T - 1 : 0;
-            CXB_LAUNCH(tc::k_hmm_tc_finish, (unsigned)B, 128, 0, stream, out + (size_t)t_last * row, tc_part[(this->T - 1) & 1].p, (int)B,
-                       bpad, K, n_slices);
-        }
-        if (tracing) {  // stamps of the LAST step kernel of the backward pass, averaged over the CTAs, relative to CTA start
-            std::vector<long long> h((size_t)tiles * n_slices * 16);
-            CXB_CUDA(cudaStreamSynchronize(stream));
-            CXB_CUDA(cudaMemcpy(h.data(), trace.p, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-            static const char* names[10] = {"start", "init+alloc done", "producer issued all", "mma: first chunk landed", "mma: last chunk landed",
-                                            "mma: all issued", "epi: prev normalised", "epi: accumulator ready", "epi: done", "exit"};
-            for (int k = 0; k < 10; ++k) {
-                double acc = 0;
-                for (int c = 0; c < tiles * n_slices; ++c) acc += (double)(h[(size_t)c * 16 + k] - h[(size_t)c * 16]);
-                fprintf(stderr, "cxb_hmm tc trace: %-26s %8.0f cycles\n", names[k], acc / (tiles * n_slices));
-            }
-        }
-        return CXB_OK;
-    }
-    int32_t launch_k64_mma() {
-        const size_t smem = (size_t)2 * 2 * 8 * 72 * 2 + (size_t)2 * 2 * 8 * 4 * 4 + 2 * 32 * 8 + (size_t)M * 64 * sizeof(float);
-        const unsigned grid = (unsigned)((B + 7) / 8);
-        const float *a = (const float*)A.p, *at = (const float*)At.p, *en = (const float*)En.p;
-        if (smem > 48 * 1024) {
-            CXB_CUDA(cudaFuncSetAttribute(k_hmm64_mma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CXB_CUDA(cudaFuncSetAttribute(k_hmm64_mma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        }
-        CXB_LAUNCH((k_hmm64_mma<true>), grid, 128, smem, stream, a, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-        CXB_LAUNCH((k_hmm64_mma<false>), grid, 128, smem, stream, at, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-        return CXB_OK;
-    }
-    // Measured alternative for K = 64, fp32 (CXB_HMM64_TC=1): both recursions in one launch on mma.sync tensor cores with
-    // three-piece bf16 operands, meeting in the middle (hmm64_tc.cuh). Parity-green, but slower than the FFMA2 register
-    // kernel below: 216 instructions per warp and step on a mostly serial dependency chain run at 0.31 instructions per
-    // cycle and scheduler with the two warps a scheduler gets (1,430 cycles per step of both recursions against
-    // 2 x 605 for the two FFMA2 passes; profiles/r02_hmm64_tc_ncu.txt).
-    int32_t launch_k64_tc() {
-        const size_t smem = h64::smem_bytes(M, true);
-        const unsigned grid = (unsigned)((B + h64::NB - 1) / h64::NB);
-        CXB_CUDA(cudaFuncSetAttribute(h64::k_hmm64_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CXB_LAUNCH((h64::k_hmm64_tc<true>), grid, 256, smem, stream, (const float*)A.p, (const float*)At.p, (const float*)En.p, obs.p,
-                   (float*)fwd.p, (float*)marg.p, B, this->T, M);
-        return CXB_OK;
-    }
     int32_t launch_k64() {
-        {
-            bool tc64 = false;
-            if (const char* e = getenv("CXB_HMM64_TC")) tc64 = atoi(e) != 0;
-            const bool other = (getenv("CXB_HMM64_MMA") && atoi(getenv("CXB_HMM64_MMA"))) || (getenv("CXB_HMM64_SPLIT") && atoi(getenv("CXB_HMM64_SPLIT")));
-            if (tc64 && !other) return launch_k64_tc();
-        }
-        // The tensor-core variant (mma.sync, 8 chains per CTA, k_hmm64_mma) is kept as a measured alternative
-        // (CXB_HMM64_MMA=1): with one 64 x 64 x 8 product per SM and step it has a single warp per scheduler and pays every
-        // latency in full — 970 cycles per step against 630 for the FFMA2 kernel below (T = 4,000: 3.94 ms vs 2.55 ms).
-        if (M <= 128 && getenv("CXB_HMM64_MMA") && atoi(getenv("CXB_HMM64_MMA"))) return launch_k64_mma();
-        {   // Two warps per chain (k_hmm64_split), a measured alternative (CXB_HMM64_SPLIT=1): it halves the FFMA2 chain of a
-            // warp but every warp repeats the per-step bookkeeping (emission, scaling, butterfly, stores) and the pair meets at
-            // a barrier, so the step is issue-bound at a HIGHER instruction count: B = 1,024, T = 1e5: 80.6 ms against 63.9 ms
-            // for one warp per chain (790 vs 630 cycles per step).
-            bool split = false;
-            if (const char* e = getenv("CXB_HMM64_SPLIT")) split = atoi(e) != 0;
-            if (split) {
-                const bool em_smem = M <= 128;
-                const size_t smem = (size_t)(2 * 72 + 8) * sizeof(float) + (em_smem ? (size_t)M * 64 * sizeof(float) : 0);
-                const float *a = (const float*)A.p, *at = (const float*)At.p, *en = (const float*)En.p;
-                const unsigned grid = (unsigned)B;
-                if (em_smem) {
-                    CXB_LAUNCH((k_hmm64_split<true, true>), grid, 64, smem, stream, a, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-                    CXB_LAUNCH((k_hmm64_split<false, true>), grid, 64, smem, stream, at, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-                } else {
-                    CXB_LAUNCH((k_hmm64_split<true, false>), grid, 64, smem, stream, a, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-                    CXB_LAUNCH((k_hmm64_split<false, false>), grid, 64, smem, stream, at, en, obs.p, (float*)fwd.p, (float*)marg.p, B, this->T, M);
-                }
-                return CXB_OK;
-            }
-        }
         // one warp per chain; warps per CTA chosen so that one CTA per SM holds the whole batch when it can (its warps
         // then spread evenly over the 4 schedulers): 1,024 chains -> 147 CTAs of 7 warps
         int n_sm = 148;
         cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
-        int wpc = (int)std::min<long long>(8, std::max<long long>(1, (B + n_sm - 1) / n_sm));
-        if (const char* e = getenv("CXB_HMM_WARPS")) wpc = std::max(1, std::min(8, atoi(e)));
+        const int wpc = (int)std::min<long long>(8, std::max<long long>(1, (B + n_sm - 1) / n_sm));
         const unsigned grid = (unsigned)((B + wpc - 1) / wpc), threads = 32u * (unsigned)wpc;
         const bool em_smem = M <= 128;
         size_t smem = (size_t)wpc * 2 * 72 * sizeof(float) + (em_smem ? (size_t)M * 64 * sizeof(float) : 0);

@@ -6,8 +6,8 @@
 // synchronisation the recursion needs):
 //   * CTA (tile, slice) owns 128 chains (MMA M) x NT = 32 or 64 output states and the full reduction over K input states;
 //   * operands are bf16 "split" pieces (x = p0 + p1 + p2, piece k = bf16 of what the earlier pieces left over); the product
-//     is accumulated in fp32 in TMEM from the piece products p_a q_b with a + b < 3 (fp32-level accuracy; NP = 2 pieces:
-//     ~2^-17 per term). The table pieces of a chunk lie one after the other in the stage, so message piece a meets table
+//     is accumulated in fp32 in TMEM from the piece products p_a q_b with a + b < 3 (fp32-level accuracy, which sparse
+//     tables need: see NP below). The table pieces of a chunk lie one after the other in the stage, so message piece a meets table
 //     pieces 0 .. NP-1-a in ONE tcgen05.mma.kind::f16 of N = (NP - a) NT: NP instructions per 16 input states instead of
 //     NP (NP + 1) / 2, into NP accumulator blocks that the epilogue adds small to large;
 //   * both operands stream through a 3-stage shared-memory ring (~180 KB in flight per SM) by 1-D bulk async copies
@@ -34,10 +34,11 @@ constexpr int M_TILE = 128;   // chains per CTA (MMA M)
 // output states per CTA (MMA N) is a template parameter NT: 64 (64 CTAs at B = 1,024, K = 512) or 32 (128 CTAs: less
 // operand ingest and half the epilogue per SM, more aggregate L2 traffic)
 constexpr int K_CHUNK = 64;   // input states per operand chunk (4 MMA K-steps of 16)
-// NP = bf16 pieces per operand: x = p0 + p1 (+ p2), p_k = bf16(residual). NP = 2 keeps ~2^-17 per term (enough for dense
-// tables, where the 512 terms of a sum average it out; NOT for sparse ones: 1e-4 on a banded matrix), NP = 3 keeps
-// ~2^-25 (fp32-level; the default). Products p_a * q_b with a + b < NP: 3 or 6 MMAs per 16 input states.
-template <int NT, int NP>
+// NP = bf16 pieces per operand: x = p0 + p1 + p2, p_k = bf16(residual), ~2^-25 per term (fp32-level). Two pieces keep
+// ~2^-17 per term: enough for dense tables, where the 512 terms of a sum average it out, NOT for sparse ones (1e-4 on a
+// banded matrix). Products p_a * q_b with a + b < NP: 6 per 16 input states.
+constexpr int NP = 3;
+template <int NT>
 struct Cfg {
     static constexpr uint32_t B_CHUNK_BYTES = NT * 64 * 2;                    // table chunk, per piece
     static constexpr uint32_t STAGE_BYTES = NP * (128 * 64 * 2) + NP * B_CHUNK_BYTES;  // message pieces + table pieces
@@ -92,16 +93,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                  "r"(bytes), "r"(bar)
                  : "memory");
 }
-// the same copy delivered to the same shared-memory offset (and signalled on the same barrier offset) of every CTA in `mask`
-__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar), "h"(mask)
-                 : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __device__ __forceinline__ uint64_t smem_desc(uint32_t addr) {  // K-major, no swizzle, version 1 (Blackwell)
     return (uint64_t)((addr & 0x3FFFFu) >> 4) | ((uint64_t)(LBO >> 4) << 16) | ((uint64_t)(SBO >> 4) << 32) | (1ull << 46);
 }
@@ -117,11 +108,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// arrive on the barrier at this offset in EVERY CTA of `mask` when the MMAs issued so far have completed
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-                 : "memory");
 }
 __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {  // no wait: several loads in flight
     asm volatile(
@@ -161,7 +147,6 @@ __device__ __forceinline__ float rcp_nr(float x) {  // MUFU.RCP + one Newton ste
     return fmaf(q, fmaf(-x, q, 1.0f), q);
 }
 // split 8 consecutive values into NP bf16 pieces (piece k = bf16 of what the earlier pieces left over), one 16-byte vector each
-template <int NP>
 __device__ __forceinline__ void split_store8(const float* x, __nv_bfloat16* const (&dst)[NP]) {
     float res[8];
 #pragma unroll
@@ -204,15 +189,10 @@ __device__ __forceinline__ void load_row64(const float* p, float4 (&v)[16]) {
     for (int i = 0; i < 16; ++i) v[i] = reinterpret_cast<const float4*>(p)[i];
 }
 
-// CL > 1: the CL CTAs that hold consecutive slices of ONE chain tile form a cluster; each loads 1 / CL of every message
-// chunk and multicasts it to all of them (the message operand is the same for every slice: 393 KB per CTA and step of
-// L2 -> SM traffic become 393 / CL KB issued per CTA; L2 read throughput, ~6,300 B/clk chip-wide, is what the ingest
-// of a step waits on). A stage may only be refilled when EVERY CTA of the cluster has consumed it: the empty barriers
-// count CL arrivals and every MMA commit arrives on the barrier of all CL CTAs.
-template <bool FWD, int NT, int NP, int CL = 1>
+template <bool FWD, int NT>
 __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
-    constexpr int N_TILE = NT, STAGES = Cfg<NT, NP>::STAGES;
-    constexpr uint32_t B_CHUNK_BYTES = Cfg<NT, NP>::B_CHUNK_BYTES, STAGE_BYTES = Cfg<NT, NP>::STAGE_BYTES, TMEM_COLS = Cfg<NT, NP>::TMEM_COLS;
+    constexpr int N_TILE = NT, STAGES = Cfg<NT>::STAGES;
+    constexpr uint32_t B_CHUNK_BYTES = Cfg<NT>::B_CHUNK_BYTES, STAGE_BYTES = Cfg<NT>::STAGE_BYTES, TMEM_COLS = Cfg<NT>::TMEM_COLS;
     constexpr int LPR = N_TILE / 4, RPI = 32 / LPR, ITER = 32 / RPI;  // lanes per row, rows per instruction, iterations per warp
     extern __shared__ __align__(128) unsigned char smem[];
     const int n_chunks = a.K / K_CHUNK;
@@ -234,7 +214,7 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
     if (threadIdx.x == 0) {
         for (int s = 0; s < STAGES; ++s) {
             mbar_init(smem_u32(&full[s]), 1);
-            mbar_init(smem_u32(&empty[s]), CL);
+            mbar_init(smem_u32(&empty[s]), 1);
         }
         mbar_init(smem_u32(accum), 2);  // both issuers commit
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -247,11 +227,6 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-    uint32_t crank = 0;
-    if (CL > 1) {
-        asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
-        cluster_sync_all();  // every CTA's barriers exist before anyone multicasts into them
-    }
     asm volatile("griddepcontrol.wait;" ::: "memory");  // everything below reads what the previous step's grid wrote
     if (threadIdx.x == 0) stamp(a, 1);
 
@@ -269,13 +244,7 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
                 // the NP pieces of a chunk are contiguous in global memory (message: [tile][chunk][piece], table: [slice][chunk][piece])
                 // and in the stage: ONE bulk copy per operand and stage. The copy engine of an SM moves a 60 KB stage at
                 // 98 B/clk as one copy but at 55 B/clk as six (profiles/r02_bulk_ingest.log) - the ingest is what a step waits on.
-                if (CL == 1) {
-                    bulk_g2s(st, op + (size_t)c * NP * (A_CHUNK_BYTES / 2), NP * A_CHUNK_BYTES, bar);
-                } else {
-                    constexpr uint32_t PART = NP * A_CHUNK_BYTES / CL;  // this CTA's share of the chunk, delivered to the whole cluster
-                    bulk_g2s_mc(st + crank * PART, op + (size_t)c * NP * (A_CHUNK_BYTES / 2) + (size_t)crank * (PART / 2), PART, bar,
-                                (uint16_t)((1u << CL) - 1u));
-                }
+                bulk_g2s(st, op + (size_t)c * NP * (A_CHUNK_BYTES / 2), NP * A_CHUNK_BYTES, bar);
                 bulk_g2s(st + NP * A_CHUNK_BYTES, tb + (size_t)c * NP * (B_CHUNK_BYTES / 2), NP * B_CHUNK_BYTES, bar);
             }
             stamp(a, 2);
@@ -286,7 +255,7 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
         // tell phases two apart) =====
         if (lane == 0) {
             const int me = warp - 5;
-            const uint32_t tmem_set = tmem_base + (uint32_t)me * Cfg<NT, NP>::SET_COLS;
+            const uint32_t tmem_set = tmem_base + (uint32_t)me * Cfg<NT>::SET_COLS;
             bool first = true;
             for (int c = 0; c < n_chunks; ++c) {
                 const int s = c % STAGES;
@@ -302,13 +271,10 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
 #pragma unroll
                     for (int pa = 0; pa < NP; ++pa)  // message piece pa x table pieces 0 .. NP-1-pa (one operand of (NP - pa) NT rows)
                         umma_bf16(tmem_set, smem_desc(a_base + pa * A_CHUNK_BYTES + off), smem_desc(b_base + off),
-                                  Cfg<NT, NP>::idesc((uint32_t)((NP - pa) * NT)), !first || (ks != 0) || (pa != 0));
+                                  Cfg<NT>::idesc((uint32_t)((NP - pa) * NT)), !first || (ks != 0) || (pa != 0));
                 }
                 first = false;
-                if (CL == 1)
-                    umma_commit(smem_u32(&empty[s]));  // frees the stage when these MMAs have read it
-                else
-                    umma_commit_mc(smem_u32(&empty[s]), (uint16_t)((1u << CL) - 1u));  // ... in every CTA that refills it
+                umma_commit(smem_u32(&empty[s]));  // frees the stage when these MMAs have read it
             }
             umma_commit(smem_u32(accum));
             if (me == 0) stamp(a, 5);
@@ -384,7 +350,7 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
                 uint32_t blkv[NP][32];
 #pragma unroll
                 for (int blk = 0; blk < NP; ++blk)
-                    tmem_ld32_issue(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)set * Cfg<NT, NP>::SET_COLS + (uint32_t)(blk * N_TILE + half * 32), blkv[blk]);
+                    tmem_ld32_issue(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)set * Cfg<NT>::SET_COLS + (uint32_t)(blk * N_TILE + half * 32), blkv[blk]);
                 tmem_ld_wait();
 #pragma unroll
                 for (int i = 0; i < 32; ++i) {
@@ -456,13 +422,8 @@ __device__ __forceinline__ void hmm_tc_step_body(const StepArgs& a) {
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (CL > 1) cluster_sync_all();  // no CTA leaves while a peer's commit may still arrive on its barriers
     if (threadIdx.x == 0) stamp(a, 9);
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
-}
-template <bool FWD, int NT, int NP>
-__global__ void __launch_bounds__(THREADS, 1) k_hmm_tc_step(const StepArgs a) {
-    hmm_tc_step_body<FWD, NT, NP>(a);
 }
 // Both passes in ONE launch per step: blockIdx.z = 0 runs step s of the forward pass (time s), blockIdx.z = 1 step s of the
 // backward pass (time T-1-s). The two recursions are independent, so a launch holds twice the CTAs (2 x 64 at B = 1,024,
@@ -473,12 +434,12 @@ __global__ void __launch_bounds__(THREADS, 1) k_hmm_tc_step(const StepArgs a) {
 struct StepArgs2 {
     StepArgs d[2];
 };
-template <int NT, int NP, int CL>
+template <int NT>
 __global__ void __launch_bounds__(THREADS, 1) k_hmm_tc_step_pair(const StepArgs2 p) {
     if (blockIdx.z == 0)
-        hmm_tc_step_body<true, NT, NP, CL>(p.d[0]);
+        hmm_tc_step_body<true, NT>(p.d[0]);
     else
-        hmm_tc_step_body<false, NT, NP, CL>(p.d[1]);
+        hmm_tc_step_body<false, NT>(p.d[1]);
 }
 // marginal rows the backward half left as normalised predictions: marg = normalise(fwd * marg), one warp per (time, chain) row
 __global__ void k_hmm_tc_combine(const float* __restrict__ fwd, float* __restrict__ marg, long long n_rows, int K) {
@@ -504,7 +465,7 @@ __global__ void k_hmm_tc_combine(const float* __restrict__ fwd, float* __restric
 }
 
 // first step of a pass: carried message = emission message; result = emission (FWD) / forward message (BWD)
-template <bool FWD, int NT, int NP>
+template <bool FWD, int NT>
 __global__ void k_hmm_tc_init(StepArgs a) {
     constexpr int N_TILE = NT;
     const int m = blockIdx.x * blockDim.x + threadIdx.x;  // chain (padded)
@@ -532,7 +493,7 @@ __global__ void k_hmm_tc_init(StepArgs a) {
 #pragma unroll
         for (int pc = 0; pc < NP; ++pc)
             dst[pc] = a.op_out + ((size_t)tile * NP * n_chunks + (size_t)(n0 / K_CHUNK) * NP + pc) * (A_CHUNK_BYTES / 2) + e;
-        split_store8<NP>(c, dst);
+        split_store8(c, dst);
     }
     a.part_out[(size_t)(0 * n_slices + slice) * a.Bpad + m] = sum_c;
     a.part_out[(size_t)(1 * n_slices + slice) * a.Bpad + m] = sum_r;
@@ -547,10 +508,10 @@ __global__ void k_hmm_tc_finish(float* raw, const float* part, int B, int Bpad, 
     for (int n = threadIdx.x; n < K; n += blockDim.x) raw[(size_t)m * K + n] *= q;
 }
 
-template <int NT, int NP>
+template <int NT>
 inline size_t step_smem_bytes(int n_sym) {
-    return (size_t)Cfg<NT, NP>::STAGES * Cfg<NT, NP>::STAGE_BYTES + (size_t)n_sym * NT * sizeof(float) +
-           (2 * Cfg<NT, NP>::STAGES + 1) * sizeof(uint64_t) + 16;
+    return (size_t)Cfg<NT>::STAGES * Cfg<NT>::STAGE_BYTES + (size_t)n_sym * NT * sizeof(float) +
+           (2 * Cfg<NT>::STAGES + 1) * sizeof(uint64_t) + 16;
 }
 
 // host: bf16 round-to-nearest-even of a float
@@ -568,19 +529,19 @@ inline float bf16_to_float_host(uint16_t h) {
     return x;
 }
 // table image: rows[n][k] (n = output state, k = input state), fp32 -> [slice][chunk][piece][NT x 64] in the canonical layout
-inline void build_table_image(const float* rows, int K, int N_TILE, int n_pieces, std::vector<uint16_t>& img) {
+inline void build_table_image(const float* rows, int K, int N_TILE, std::vector<uint16_t>& img) {
     const int n_chunks = K / K_CHUNK, n_slices = K / N_TILE;
     const size_t B_CHUNK_BYTES = (size_t)N_TILE * K_CHUNK * 2;
-    img.assign((size_t)n_slices * n_pieces * n_chunks * (B_CHUNK_BYTES / 2), 0);
+    img.assign((size_t)n_slices * NP * n_chunks * (B_CHUNK_BYTES / 2), 0);
     for (int n = 0; n < K; ++n)
         for (int k = 0; k < K; ++k) {
             float res = rows[(size_t)n * K + k];
             const int slice = n / N_TILE, r = n % N_TILE, c = k / K_CHUNK, kk = k % K_CHUNK;
-            const size_t base = (size_t)slice * n_pieces * n_chunks * (B_CHUNK_BYTES / 2);
-            for (int pc = 0; pc < n_pieces; ++pc) {
+            const size_t base = (size_t)slice * NP * n_chunks * (B_CHUNK_BYTES / 2);
+            for (int pc = 0; pc < NP; ++pc) {
                 const uint16_t piece = bf16_rn_host(res);
                 res -= bf16_to_float_host(piece);
-                img[base + (size_t)(c * n_pieces + pc) * (B_CHUNK_BYTES / 2) + chunk_elem(r, kk)] = piece;
+                img[base + (size_t)(c * NP + pc) * (B_CHUNK_BYTES / 2) + chunk_elem(r, kk)] = piece;
             }
         }
 }

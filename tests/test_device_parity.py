@@ -436,11 +436,12 @@ def _hmm_numpy(A, E, obs):
     return fwd, marg
 
 
-@pytest.mark.parametrize("T,M", [(1, 3), (2, 3), (3, 3), (4, 5), (5, 5), (9, 32), (70, 100), (3000, 32)])
-def test_hmm64_kernel_lengths_and_long_chain_vs_numpy(T, M):
-    """K = 64 fp32 register kernel: the two-step-late write-out (T around the pipeline depth), emission tables in shared
-    memory (M <= 64) and in global memory, and the drift-free power-of-two scaling over a long chain."""
-    B, K = 5, 64
+@pytest.mark.parametrize("B,T,M", [(5, 1, 3), (5, 2, 3), (5, 3, 3), (5, 4, 5), (5, 5, 5), (5, 9, 32), (5, 70, 100), (5, 3000, 32),
+                                   (1, 1, 3), (4, 301, 200)])
+def test_hmm64_kernel_lengths_and_long_chain_vs_numpy(B, T, M):
+    """K = 64 fp32 register kernel: the late write-out (T around the pipeline depth), a single chain, emission tables in
+    shared memory (M <= 128) and in global memory (M = 200), and the drift-free power-of-two scaling over a long chain."""
+    K = 64
     rng = np.random.Generator(np.random.PCG64(77))
     A = rng.dirichlet(np.ones(K) * 0.3, size=K)
     E = rng.dirichlet(np.ones(K) * 0.5, size=M).T * K
@@ -459,23 +460,17 @@ def test_hmm64_kernel_lengths_and_long_chain_vs_numpy(T, M):
         np.testing.assert_allclose(got_m[:, b, :].sum(axis=-1), 1.0, rtol=0, atol=2e-6)
 
 
+# The slice width follows the grid: 32 output states per CTA while (chain tiles) x (K / 32) x 2 CTAs fit one per SM,
+# else 64. On a 148-SM B200 the last five shapes are the ones that get NT = 64 (5 x 16 x 2 = 160, 3 x 32 x 2 = 192,
+# 14 x 6 x 2 = 168 and 9 x 10 x 2 = 180 CTAs): T = 1 and 2 for the hand-over, and K / 64 odd.
 @pytest.mark.parametrize("K,B,T,M", [(128, 5, 1, 4), (128, 5, 2, 4), (128, 130, 3, 7), (256, 7, 6, 32), (512, 131, 5, 32),
-                                      (512, 3, 40, 64), (320, 9, 12, 5), (512, 2, 1200, 16), (192, 3, 700, 9)])
-@pytest.mark.parametrize("schedule", ["paired", "pass_after_pass", "paired_nt64", "two_pieces", "cluster4", "cluster8"])
-def test_hmm_tensor_core_kernel_vs_numpy(K, B, T, M, schedule, monkeypatch):
-    """K >= 128 fp32: tcgen05 path (bf16 split operands, fp32 TMEM accumulators, one launch per time step), ragged chain
-    tiles (B not a multiple of 128), every pipeline depth, against the dense fp64 forward-backward. Schedules: both passes
-    in one launch per step (default; T = 1, 2, 3 exercise the hand-over between stored predictions and direct marginals),
-    one pass after the other, the 64-state slice variant, the 2-piece operand split, and thread-block clusters with a
-    multicast message operand."""
-    if schedule == "pass_after_pass":
-        monkeypatch.setenv("CXB_HMM_TC_PAIRED", "0")
-    elif schedule == "paired_nt64":
-        monkeypatch.setenv("CXB_HMM_TC_NT", "64")
-    elif schedule == "two_pieces":
-        monkeypatch.setenv("CXB_HMM_TC_PIECES", "2")
-    elif schedule in ("cluster4", "cluster8"):  # slices of a chain tile in one cluster, message operand multicast (when the slices divide)
-        monkeypatch.setenv("CXB_HMM_TC_CLUSTER", schedule[-1])
+                                      (512, 3, 40, 64), (320, 9, 12, 5), (512, 2, 1200, 16), (192, 3, 700, 9),
+                                      (512, 600, 5, 16), (1024, 300, 3, 8), (512, 600, 2, 16), (192, 1700, 1, 4),
+                                      (320, 1100, 2, 5)])
+def test_hmm_tensor_core_kernel_vs_numpy(K, B, T, M):
+    """K >= 128 fp32: tcgen05 path (bf16 split operands, fp32 TMEM accumulators, one launch per time step running both
+    passes), ragged chain tiles (B not a multiple of 128), every pipeline depth, both slice widths, against the dense fp64
+    forward-backward. T = 1, 2, 3 exercise the hand-over between stored predictions and direct marginals."""
     rng = np.random.Generator(np.random.PCG64(2024 + K))
     A = rng.dirichlet(np.ones(K) * 0.5, size=K)
     E = rng.dirichlet(np.ones(K) * 0.5, size=M).T * K
@@ -510,76 +505,6 @@ def test_hmm_tensor_core_kernel_matches_simt_kernel(monkeypatch):
         res.append((hm.get_forward(), hm.get_marginals()))
     assert_close(res[0][0], res[1][0], cap.F32)
     assert_close(res[0][1], res[1][1], cap.F32)
-
-
-@pytest.mark.parametrize("B,T,M", [(1, 1, 3), (3, 2, 3), (5, 7, 4), (19, 37, 32), (8, 130, 100), (4, 300, 200)])
-def test_hmm64_two_warps_per_chain_variant_vs_numpy(B, T, M, monkeypatch):
-    """k_hmm64_split (CXB_HMM64_SPLIT=1): two warps per chain exchanging through shared memory; same tolerance as the default."""
-    monkeypatch.setenv("CXB_HMM64_SPLIT", "1")
-    K = 64
-    rng = np.random.Generator(np.random.PCG64(77 + T))
-    A = rng.dirichlet(np.ones(K), size=K)
-    E = rng.dirichlet(np.ones(K), size=M).T * K
-    obs = rng.integers(0, M, size=(T, B)).astype(np.uint8)
-    hm = C.HmmBatch(B, T, K, M, dtype=cap.F32)
-    hm.set_tables(A, E)
-    hm.set_observations(obs)
-    hm.update_marginals()
-    got_m, got_f = hm.get_marginals(), hm.get_forward()
-    A_used = A.astype(np.float32).astype(np.float64)
-    for b in (0, B - 1):
-        want_f, want_m = _hmm_numpy(A_used, E, obs[:, b])
-        assert_close(got_f[:, b, :], want_f, cap.F32)
-        assert_close(got_m[:, b, :], want_m, cap.F32)
-
-
-@pytest.mark.parametrize("B,T,M", [(5, 3, 4), (19, 37, 32), (8, 130, 100)])
-def test_hmm64_tensor_core_variant_vs_numpy(B, T, M, monkeypatch):
-    """The mma.sync variant of the K = 64 kernel (CXB_HMM64_MMA=1; measured slower than the FFMA2 kernel, kept as evidence
-    for the K threshold of the tensor-core path) against the dense fp64 forward-backward."""
-    monkeypatch.setenv("CXB_HMM64_MMA", "1")
-    K = 64
-    rng = np.random.Generator(np.random.PCG64(31))
-    A = rng.dirichlet(np.ones(K) * 0.4, size=K)
-    E = rng.dirichlet(np.ones(K) * 0.5, size=M).T * K
-    obs = rng.integers(0, M, size=(T, B)).astype(np.uint8)
-    hm = C.HmmBatch(B, T, K, M, dtype=cap.F32)
-    hm.set_tables(A, E)
-    hm.set_observations(obs)
-    hm.update_marginals()
-    got_m, got_f = hm.get_marginals(), hm.get_forward()
-    A_used = A.astype(np.float32).astype(np.float64)
-    for b in (0, B - 1):
-        want_f, want_m = _hmm_numpy(A_used, E, obs[:, b])
-        # NOT the product path: this experimental variant splits its operands into two bf16 pieces (2^-17 per term), so it is
-        # held to 2e-5 element-wise; the default K = 64 kernel (fp32 FFMA) is held to the north-star 1e-5 above
-        np.testing.assert_allclose(got_f[:, b, :], want_f, rtol=2e-5, atol=1e-8)
-        np.testing.assert_allclose(got_m[:, b, :], want_m, rtol=2e-5, atol=1e-8)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("B,T,M", [(1, 1, 3), (3, 2, 3), (5, 3, 4), (8, 4, 4), (9, 5, 7), (19, 37, 32), (8, 130, 100), (4, 301, 200), (11, 3000, 32)])
-def test_hmm64_both_recursions_on_tensor_cores_variant_vs_numpy(B, T, M, monkeypatch):
-    """k_hmm64_tc (CXB_HMM64_TC=1, hmm64_tc.cuh): forward and backward recursion of 8 chains in one CTA on mma.sync with
-    three-piece bf16 operands, meeting in the middle (T odd / even, T below the pipeline depth, ragged chain groups, the
-    two-step-delayed damped scaling over a long chain). Held to the north-star tolerance like the default kernel."""
-    monkeypatch.setenv("CXB_HMM64_TC", "1")
-    K = 64
-    rng = np.random.Generator(np.random.PCG64(91 + T))
-    A = rng.dirichlet(np.ones(K) * 0.3, size=K)
-    E = rng.dirichlet(np.ones(K) * 0.5, size=M).T * K
-    obs = rng.integers(0, M, size=(T, B)).astype(np.uint8)
-    hm = C.HmmBatch(B, T, K, M, dtype=cap.F32)
-    hm.set_tables(A, E)
-    hm.set_observations(obs)
-    assert hm.update_marginals() == B * (6 * T - 4)
-    got_m, got_f = hm.get_marginals(), hm.get_forward()
-    A_used = A.astype(np.float32).astype(np.float64)
-    for b in sorted({0, B // 2, B - 1}):
-        want_f, want_m = _hmm_numpy(A_used, E, obs[:, b])
-        assert_close(got_f[:, b, :], want_f, cap.F32)
-        assert_close(got_m[:, b, :], want_m, cap.F32)
-        np.testing.assert_allclose(got_m[:, b, :].sum(axis=-1), 1.0, rtol=0, atol=2e-6)
 
 
 def _pairwise_vs_oracle(oracle_api, dtype, n, edges, K, sweeps, seed=7):
