@@ -13,8 +13,14 @@
 // shared-memory line and read back with broadcast 128-bit loads, so a step is K*K/32 FFMAs + K/4 LDS per warp
 // and no block-level barrier.  Larger K stream Tbl through shared memory in row tiles shared by the 8 chains of
 // the CTA.
-// Which kernel runs: K = 64 fp32 -> k_hmm64_pass; fp32, K >= 128 a multiple of 64, M <= 64 -> the tcgen05 path of
-// hmm_tc.cuh (k_hmm_tc_step_pair); every other (K, dtype), and CXB_HMM_NO_TC=1 -> k_hmm_pass.
+// Which kernel runs (Hmm::launch_t; tests/test_hmm_widths.py keeps a copy of the rule):
+//   * fp32, K = 64 -> k_hmm64_pass, the emission table in shared memory for M <= 128, else read from global memory;
+//   * fp32, K >= 128 a multiple of 64, M <= 64 -> the tcgen05 path of hmm_tc.cuh (k_hmm_tc_step_pair<NT>, NT = 32 or 64);
+//   * K = 32 -> k_hmm_pass with the table in registers;
+//   * every other (K, dtype, M), and CXB_HMM_NO_TC=1 -> k_hmm_pass with the table in shared memory: whole when it fits,
+//     else streamed in row tiles; the emission table sits in shared memory when it and one table row fit in 200 KiB next
+//     to the staging, else in global memory.  Every shape cxb_hmm_create accepts (2 <= K <= 1024, 1 <= M <= 256) runs.
+// cxb_hmm_set_observations refuses a symbol >= M, so the kernels' clamp of o to M - 1 never changes a value.
 #include <algorithm>
 #include <cmath>
 #include <type_traits>
@@ -39,10 +45,11 @@ __device__ __forceinline__ T warp_sum(T v) {
 // BWD: t descending, reads fwd[t], writes marg[t] = normalise(fwd[t] * bwd_t), carries
 // m2f(z_t, tr_{t-1}) = normalise(em_t * bwd_t).  tbl is A (FWD) or A^T (BWD), row-major [K][K];
 // emis_n is the column-normalised emission table transposed to [M][K] (m2v(z_t, em_t) = emis_n[o_t]), staged in
-// shared memory.  Nothing on the per-step critical path waits on global memory: observations are fetched 32 steps at a
+// shared memory (EM_SMEM) or, when it does not fit next to a table row, read from global memory (<= 2 MB, L2-resident).
+// Nothing on the per-step critical path waits on global memory: observations are fetched 32 steps at a
 // time (one per lane, broadcast by shuffle, double buffered), the forward message of the next step is already in
 // registers and the one 8 steps ahead is being pulled into L2 (prefetch.global.L2).
-template <class T, int K, bool REGA, bool FWD>
+template <class T, int K, bool REGA, bool FWD, bool EM_SMEM>
 __global__ void __launch_bounds__(HMM_WARPS * 32)
 k_hmm_pass(const T* __restrict__ tbl, const T* __restrict__ emis_n, const uint8_t* __restrict__ obs, T* __restrict__ fwd,
            T* __restrict__ marg, long long B, long long Tn, int Kdyn, int n_sym, int tile_rows) {
@@ -55,8 +62,8 @@ k_hmm_pass(const T* __restrict__ tbl, const T* __restrict__ emis_n, const uint8_
     const bool live = b < B;
     const long long bb = live ? b : 0;
     T* sh_v = reinterpret_cast<T*>(smem_raw) + (size_t)warp * Kk;            // per-warp staging of v
-    T* sh_em = reinterpret_cast<T*>(smem_raw) + (size_t)HMM_WARPS * Kk;        // [M][K] emission messages
-    T* sh_tbl = sh_em + (size_t)n_sym * Kk;                                    // streamed path: row tile of tbl
+    T* sh_em = reinterpret_cast<T*>(smem_raw) + (size_t)HMM_WARPS * Kk;        // [M][K] emission messages (EM_SMEM)
+    T* sh_tbl = sh_em + (EM_SMEM ? (size_t)n_sym * Kk : 0);                    // streamed path: row tile of tbl
 
     T areg[REGA ? K : 1][REGA ? K / 32 : 1];
     if (REGA) {
@@ -65,7 +72,8 @@ k_hmm_pass(const T* __restrict__ tbl, const T* __restrict__ emis_n, const uint8_
 #pragma unroll
             for (int c = 0; c < K / 32; ++c) areg[i][c] = tbl[(size_t)i * K + lane + 32 * c];
     }
-    for (int x = threadIdx.x; x < n_sym * Kk; x += blockDim.x) sh_em[x] = emis_n[x];
+    if (EM_SMEM)
+        for (int x = threadIdx.x; x < n_sym * Kk; x += blockDim.x) sh_em[x] = emis_n[x];
     const bool whole_table = !REGA && tile_rows >= Kk;
     if (whole_table)
         for (int x = threadIdx.x; x < Kk * Kk; x += blockDim.x) sh_tbl[x] = tbl[x];
@@ -173,12 +181,12 @@ k_hmm_pass(const T* __restrict__ tbl, const T* __restrict__ emis_n, const uint8_
                 }
             }
         }
-        // emission message of this step (shared memory)
+        // emission message of this step
         T em[CPL_MAX];
 #pragma unroll
         for (int c = 0; c < CPL_MAX; ++c) {
             int j = lane + 32 * c;
-            em[c] = (c < cpl && j < Kk) ? sh_em[(size_t)o * Kk + j] : T(0);
+            em[c] = (c < cpl && j < Kk) ? (EM_SMEM ? sh_em[(size_t)o * Kk + j] : __ldg(&emis_n[(size_t)o * Kk + j])) : T(0);
         }
         const size_t base = ((size_t)t * B + bb) * Kk;
         if (FWD) {
@@ -387,6 +395,20 @@ k_hmm64_pass(const float* __restrict__ tbl, const float* __restrict__ emis_n, co
     }
 }
 
+// cxb_hmm_set_observations' range check: *bad = 1 if any of the n bytes is >= n_sym (< 256). Four bytes per compare
+// (__vcmpgeu4), 16 per load; cudaMalloc'd obs is 16-byte aligned, the last n % 16 bytes are read one by one.
+__global__ void __launch_bounds__(256) k_hmm_check_obs(const uint8_t* __restrict__ obs, size_t n, int n_sym, int* __restrict__ bad) {
+    const unsigned lim = 0x01010101u * (unsigned)n_sym;
+    const size_t n16 = n / 16, stride = (size_t)gridDim.x * blockDim.x, tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned any = 0;
+    for (size_t i = tid; i < n16; i += stride) {
+        const uint4 w = __ldg(reinterpret_cast<const uint4*>(obs) + i);
+        any |= __vcmpgeu4(w.x, lim) | __vcmpgeu4(w.y, lim) | __vcmpgeu4(w.z, lim) | __vcmpgeu4(w.w, lim);
+    }
+    for (size_t i = n16 * 16 + tid; i < n; i += stride) any |= obs[i] >= n_sym;
+    if (__syncthreads_or(any != 0) && threadIdx.x == 0) *bad = 1;
+}
+
 struct Hmm {
     int device = 0, dtype = CXB_F32, K = 0, M = 0;
     long long B = 0, T = 0;
@@ -395,6 +417,7 @@ struct Hmm {
     std::string err;
     DBuf<unsigned char> A, At, En, fwd, marg;
     DBuf<uint8_t> obs;
+    DBuf<int> obs_bad;  // flag of k_hmm_check_obs
     // tensor-core path (hmm_tc.cuh): table images (forward: rows of A^T, backward: rows of A), message operands, row sums
     DBuf<uint16_t> tc_img_f, tc_img_b, tc_op[2], tc_op_b[2];  // _b: the backward pass's own ping-pong
     DBuf<float> tc_part[2], tc_part_b[2];
@@ -431,6 +454,7 @@ struct Hmm {
         CXB_CUDA(At.reserve((size_t)K * K * esz()));
         CXB_CUDA(En.reserve((size_t)M * K * esz()));
         CXB_CUDA(obs.reserve((size_t)T * B));
+        CXB_CUDA(obs_bad.reserve(1));
         CXB_CUDA(fwd.reserve((size_t)T * B * K * esz()));
         CXB_CUDA(marg.reserve((size_t)T * B * K * esz()));
         return CXB_OK;
@@ -493,16 +517,16 @@ struct Hmm {
         have_tables = true;
         return CXB_OK;
     }
-    template <class T, int KK, bool REGA>
+    template <class T, int KK, bool REGA, bool EM_SMEM>
     int32_t launch_pair(int tile_rows, size_t smem) {
         unsigned grid = cdiv((size_t)B, HMM_WARPS);
         if (smem > 48 * 1024) {
-            CXB_CUDA(cudaFuncSetAttribute(k_hmm_pass<T, KK, REGA, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CXB_CUDA(cudaFuncSetAttribute(k_hmm_pass<T, KK, REGA, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CXB_CUDA(cudaFuncSetAttribute(k_hmm_pass<T, KK, REGA, true, EM_SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CXB_CUDA(cudaFuncSetAttribute(k_hmm_pass<T, KK, REGA, false, EM_SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         }
-        CXB_LAUNCH((k_hmm_pass<T, KK, REGA, true>), grid, HMM_WARPS * 32, smem, stream, (const T*)A.p, (const T*)En.p, obs.p,
+        CXB_LAUNCH((k_hmm_pass<T, KK, REGA, true, EM_SMEM>), grid, HMM_WARPS * 32, smem, stream, (const T*)A.p, (const T*)En.p, obs.p,
                    (T*)fwd.p, (T*)marg.p, B, this->T, K, M, tile_rows);
-        CXB_LAUNCH((k_hmm_pass<T, KK, REGA, false>), grid, HMM_WARPS * 32, smem, stream, (const T*)At.p, (const T*)En.p, obs.p,
+        CXB_LAUNCH((k_hmm_pass<T, KK, REGA, false, EM_SMEM>), grid, HMM_WARPS * 32, smem, stream, (const T*)At.p, (const T*)En.p, obs.p,
                    (T*)fwd.p, (T*)marg.p, B, this->T, K, M, tile_rows);
         return CXB_OK;
     }
@@ -619,17 +643,18 @@ struct Hmm {
     }
     template <class T>
     int32_t launch_t() {
-        size_t stage = ((size_t)HMM_WARPS * K + (size_t)M * K) * sizeof(T);  // per-warp staging + emission messages
+        const long long stage = (long long)HMM_WARPS * K * sizeof(T), em = (long long)M * K * sizeof(T),  // per-warp staging, emission messages
+            row = (long long)K * sizeof(T), budget = 200 * 1024;
         if (sizeof(T) == 4 && K == 64) return launch_k64();
         if (sizeof(T) == 4 && tc_ready && tc_eligible()) return launch_tc();
-        if (K == 32) return launch_pair<T, 32, true>(0, stage);
-        size_t budget = 200 * 1024 - stage;
-        int tile_rows = (int)std::min<size_t>((size_t)K, budget / ((size_t)K * sizeof(T)));
-        if (tile_rows < 1) {
-            err = "state count too large";
-            return CXB_ERR_BAD_ARG;
-        }
-        return launch_pair<T, 0, false>(tile_rows, stage + (size_t)tile_rows * K * sizeof(T));
+        if (K == 32) return launch_pair<T, 32, true, true>(0, (size_t)(stage + em));  // at most 66 KB (fp64, M = 256)
+        // the emission table stays in shared memory while it and one table row fit; else it is read from global memory (L2)
+        // and the row tiles get all but the staging: at K = 1024 fp64 that is 17 rows
+        const bool em_smem = stage + em + row <= budget;
+        const long long rest = budget - stage - (em_smem ? em : 0);
+        const int tile_rows = (int)std::min<long long>(K, rest / row);
+        const size_t smem = (size_t)(budget - rest + tile_rows * row);
+        return em_smem ? launch_pair<T, 0, false, true>(tile_rows, smem) : launch_pair<T, 0, false, false>(tile_rows, smem);
     }
     int32_t launch() {
         if (!have_tables || !have_obs) {
@@ -694,9 +719,22 @@ int32_t cxb_hmm_set_tables(cxb_hmm* m, const double* transition, const double* e
 } CXB_ABI_CATCH(CXB_ERR_INTERNAL)
 int32_t cxb_hmm_set_observations(cxb_hmm* m, const uint8_t* obs_host) try {
     Hmm* h = HM(m);
+    const size_t n = (size_t)h->T * h->B;
     HM_CUDA(m, cudaSetDevice(h->device));
-    HM_CUDA(m, cudaMemcpyAsync(h->obs.p, obs_host, (size_t)h->T * h->B, cudaMemcpyHostToDevice, h->stream));
+    h->have_obs = false;
+    HM_CUDA(m, cudaMemcpyAsync(h->obs.p, obs_host, n, cudaMemcpyHostToDevice, h->stream));
+    int bad = 0;
+    if (h->M < 256) {  // with 256 symbols every byte is one
+        HM_CUDA(m, cudaMemsetAsync(h->obs_bad.p, 0, sizeof(int), h->stream));
+        CXB_LAUNCH(cxb::k_hmm_check_obs, std::min(cxb::cdiv(n, 16 * 256), 1024u), 256, 0, h->stream, h->obs.p, n, h->M, h->obs_bad.p);
+        HM_CUDA(m, cudaGetLastError());
+        HM_CUDA(m, cudaMemcpyAsync(&bad, h->obs_bad.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    }
     HM_CUDA(m, cudaStreamSynchronize(h->stream));
+    if (bad) {
+        h->err = "observation symbol out of range (0 <= o < n_symbols)";
+        return CXB_ERR_BAD_ARG;
+    }
     h->have_obs = true;
     return CXB_OK;
 } CXB_ABI_CATCH(CXB_ERR_INTERNAL)

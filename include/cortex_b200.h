@@ -389,7 +389,8 @@ void cxb_hmm_destroy(cxb_hmm* m);
 const char* cxb_hmm_last_error(cxb_hmm* m);
 /* transition A[K][K] (row = from state), emission E[K][M]; float64 host arrays */
 int32_t cxb_hmm_set_tables(cxb_hmm* m, const double* transition, const double* emission);
-/* observations o[T][B] uint8, host */
+/* observations o[T][B] uint8, host. Every symbol must satisfy 0 <= o < n_symbols: otherwise CXB_ERR_BAD_ARG, and the
+ * handle has no observations until a later call succeeds (cxb_hmm_update_marginals returns CXB_ERR_STATE). */
 int32_t cxb_hmm_set_observations(cxb_hmm* m, const uint8_t* obs_host);
 int32_t cxb_hmm_update_marginals(cxb_hmm* m, int64_t* n_updates_out);
 /* marginals [T][B][K] engine dtype, D2H (t0..t1 slice to bound the copy) */

@@ -463,10 +463,12 @@ def test_hmm64_kernel_lengths_and_long_chain_vs_numpy(B, T, M):
 # The slice width follows the grid: 32 output states per CTA while (chain tiles) x (K / 32) x 2 CTAs fit one per SM,
 # else 64. On a 148-SM B200 the last five shapes are the ones that get NT = 64 (5 x 16 x 2 = 160, 3 x 32 x 2 = 192,
 # 14 x 6 x 2 = 168 and 9 x 10 x 2 = 180 CTAs): T = 1 and 2 for the hand-over, and K / 64 odd.
-@pytest.mark.parametrize("K,B,T,M", [(128, 5, 1, 4), (128, 5, 2, 4), (128, 130, 3, 7), (256, 7, 6, 32), (512, 131, 5, 32),
-                                      (512, 3, 40, 64), (320, 9, 12, 5), (512, 2, 1200, 16), (192, 3, 700, 9),
-                                      (512, 600, 5, 16), (1024, 300, 3, 8), (512, 600, 2, 16), (192, 1700, 1, 4),
-                                      (320, 1100, 2, 5)])
+HMM_TC_SHAPES = [(128, 5, 1, 4), (128, 5, 2, 4), (128, 130, 3, 7), (256, 7, 6, 32), (512, 131, 5, 32), (512, 3, 40, 64),
+                 (320, 9, 12, 5), (512, 2, 1200, 16), (192, 3, 700, 9), (512, 600, 5, 16), (1024, 300, 3, 8),
+                 (512, 600, 2, 16), (192, 1700, 1, 4), (320, 1100, 2, 5)]
+
+
+@pytest.mark.parametrize("K,B,T,M", HMM_TC_SHAPES)
 def test_hmm_tensor_core_kernel_vs_numpy(K, B, T, M):
     """K >= 128 fp32: tcgen05 path (bf16 split operands, fp32 TMEM accumulators, one launch per time step running both
     passes), ragged chain tiles (B not a multiple of 128), every pipeline depth, both slice widths, against the dense fp64
