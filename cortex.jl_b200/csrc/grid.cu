@@ -11,11 +11,14 @@
 //                linked m2f(v,f)  = normalise(unary * prod_{g != f} m2v(v,g))
 // Potts table psi[a][b] = exp(beta [a==b])  =>  sum_b psi[a][b] m[b] = sum(m) + (e^beta - 1) m[a].
 //
-// Kernel: fused per-pixel pass, HBM-bound (640 B of traffic per interior pixel at K=16 fp32: read 4 m2f + unary, write
-// 4 m2f + marginal).  Every m2v is computed, but only rows 0 and H - 1 store theirs: the others are a function of this
-// sweep's input m2f, which stays intact until the next sweep, so k_potts_m2v rebuilds them bit for bit on the first read
-// of an m2v plane (cxb_grid_get_messages).  No later sweep reads them; storing them would add 256 B per pixel.
-// CXB_GRID_EAGER_M2V=1 stores every m2v every sweep (896 B per pixel).  LP = K / (16 B / sizeof(T)) lanes cooperate on one
+// Kernel: fused per-pixel pass, HBM-bound (576 B of traffic per interior pixel at K=16 fp32: read 4 m2f + unary, write
+// 4 m2f).  Every m2v and every marginal is computed, but only rows 0 and H - 1 store theirs: the others are a function of
+// this sweep's input m2f and unary, which stay intact until the next sweep (or until the host flushes them before a reset,
+// set_unary or infer_host overwrites them), so k_potts_m2v rebuilds them bit for bit on the first read of an m2v plane
+// (cxb_grid_get_messages) or of the marginals (cxb_grid_get_marginals): interior-row marginals are computed only when read.
+// No later sweep reads them; storing them would add 256 B (m2v) + 64 B (marginal) per pixel.  The last sweep of an
+// infer_host job stores every marginal, so its download needs no rebuild.  CXB_GRID_EAGER_M2V=1 stores every m2v and every
+// marginal every sweep (896 B per pixel).  LP = K / (16 B / sizeof(T)) lanes cooperate on one
 // pixel, each lane moving 16-byte vectors, so a warp touches 32*16 = 512 contiguous bytes per plane per
 // instruction; K-sums are 2-4 warp-shuffle steps.  m2f planes are double buffered (sweep reads `cur`, writes
 // `nxt`), every value is read exactly once.  Row sharding: the up/down messages of the first/last local row
@@ -102,12 +105,34 @@ __device__ __forceinline__ void potts_m2v(const T (&in)[E], bool ex, T w, T (&mv
     }
 }
 
+// final phase, marginal(v) = normalise(unary * prod_f m2v(v, f)) in ascending factor order, absent factors skipped; stored at
+// marg + o when `store`. Every lane shuffles whether it stores or not. The sweep and k_potts_m2v both call this, so a rebuilt
+// marginal is bit-identical to the one the sweep would have stored.
+template <class T, int E, int LP>
+__device__ __forceinline__ void potts_marginal(const T (&un)[E], const T (&mv)[4][E], const bool (&ex)[4], bool store, void* marg, size_t o) {
+    T acc[E];
+#pragma unroll
+    for (int k = 0; k < E; ++k) {
+        T a = un[k];
+        if (ex[0]) a = a * mv[0][k];
+        if (ex[1]) a = a * mv[1][k];
+        if (ex[2]) a = a * mv[2][k];
+        if (ex[3]) a = a * mv[3][k];
+        acc[k] = a;
+    }
+    const T inv_tot = rcp_pos<T>(group_sum<T, E, LP>(acc));
+#pragma unroll
+    for (int k = 0; k < E; ++k) acc[k] = acc[k] * inv_tot;
+    if (store) store_vec<T, E>((T*)marg + o, acc);
+}
+
 struct GridView {
     long long H, W;
     int has_up, has_down;
-    // 1: store every m2v plane (CXB_GRID_EAGER_M2V=1). 0: store only rows 0 and H - 1, whose up / down inputs may come from
-    // a halo buffer that a neighbour can overwrite before the planes are read; k_potts_m2v rebuilds the other rows on read
-    int eager_m2v;
+    // The rows 1 .. H - 2 of the m2v planes / of the marginals. k_potts_sweep: 1 = store them; 0 = store only rows 0 and
+    // H - 1, whose up / down inputs may come from a halo buffer that a neighbour can overwrite before they are read, and
+    // leave the others to k_potts_m2v. k_potts_m2v: 1 = rebuild them.
+    int inner_m2v, inner_marg;
     const void* unary;       // [H][W][K]
     const void* m2f_cur[4];  // [H][W][K] per direction (message from the pixel towards direction d)
     void* m2f_nxt[4];
@@ -163,29 +188,15 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
         }
     }
     // loop phase
-    const bool store_mv = valid && (g.eager_m2v || i == 0 || i + 1 == g.H);
+    // rows 0 and H - 1 (every row when H <= 2) in one unsigned compare; i == 0 || i + 1 == g.H costs the fp32 sweep registers
+    const bool edge_row = (unsigned long long)(pix - g.W) >= (unsigned long long)(npix - 2 * g.W);
     T mv[4][E];
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
-        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], store_mv, g.m2v[d], o);
+        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], valid && (g.inner_m2v || edge_row), g.m2v[d], o);
     }
-    // final phase: marginal, then the linked m2f (products in ascending factor order, left to right)
-    {
-        T acc[E];
-#pragma unroll
-        for (int k = 0; k < E; ++k) {
-            T a = un[k];
-            if (ex[0]) a = a * mv[0][k];
-            if (ex[1]) a = a * mv[1][k];
-            if (ex[2]) a = a * mv[2][k];
-            if (ex[3]) a = a * mv[3][k];
-            acc[k] = a;
-        }
-        const T inv_tot = rcp_pos<T>(group_sum<T, E, LP>(acc));
-#pragma unroll
-        for (int k = 0; k < E; ++k) acc[k] = acc[k] * inv_tot;
-        if (valid) store_vec<T, E>((T*)g.marg + o, acc);
-    }
+    // final phase: the linked m2f, then the marginal (products in ascending factor order, left to right; the marginal last
+    // keeps the fp32 sweep at 48 registers)
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
         T acc[E];
@@ -206,12 +217,14 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
         if (d == 0 && valid && i == 0 && g.peer_up) store_vec<T, E>((T*)g.peer_up + (size_t)j * K + (size_t)lane * E, acc);
         if (d == 3 && valid && i + 1 == g.H && g.peer_down) store_vec<T, E>((T*)g.peer_down + (size_t)j * K + (size_t)lane * E, acc);
     }
+    potts_marginal<T, E, LP>(un, mv, ex, valid && (g.inner_marg || edge_row), g.marg, o);
 }
 
-// The m2v planes of rows 1 .. H - 2, which a sweep with eager_m2v == 0 does not store, rebuilt from the m2f planes that sweep
-// read (g.m2f_cur): they stay intact until the next sweep, whose own m2v supersede these. Rows 1 .. H - 2 take their up and
-// down inputs from this shard's planes, never from a halo buffer. Lane layout as in k_potts_sweep; no store where the factor
-// is absent, so those slots keep the zeros of init.
+// Rows 1 .. H - 2 of the m2v planes (g.inner_m2v) and / or of the marginals (g.inner_marg), which a sweep with the same flag
+// 0 does not store, rebuilt from the m2f planes that sweep read (g.m2f_cur) and, for the marginals, the unary plane it read
+// (g.unary): both stay intact until the next sweep, whose own values supersede these, or until the host flushes (reset,
+// set_unary, infer_host). Rows 1 .. H - 2 take their up and down inputs from this shard's planes, never from a halo buffer.
+// Lane layout as in k_potts_sweep; no m2v store where the factor is absent, so those slots keep the zeros of init.
 template <class T, int K, int E>
 __global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
     constexpr int LP = K / E;
@@ -230,7 +243,7 @@ __global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
     src[1] = (const T*)g.m2f_cur[2] + o - K;
     src[2] = (const T*)g.m2f_cur[1] + o + K;
     src[3] = (const T*)g.m2f_cur[0] + o + (size_t)g.W * K;
-    T in[4][E];  // all four loads in flight before the first store
+    T in[4][E], un[E];  // all loads in flight before the first store
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
         if (ex[d]) {
@@ -240,11 +253,13 @@ __global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
             for (int k = 0; k < E; ++k) in[d][k] = T(1);
         }
     }
+    if (g.inner_marg) load_vec<T, E>((const T*)g.unary + o, un);
+    T mv[4][E];
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
-        T mv[E];
-        potts_m2v<T, E, LP>(in[d], ex[d], w, mv, valid, g.m2v[d], o);
+        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], valid && g.inner_m2v, g.m2v[d], o);
     }
+    if (g.inner_marg) potts_marginal<T, E, LP>(un, mv, ex, valid, g.marg, o);
 }
 
 // stream-ordered hand-shake of the fused halo exchange: sweeps completed by the neighbours are counted in flags that
@@ -302,9 +317,14 @@ struct Grid {
     unsigned long long job_no = 0;
     unsigned sweep_no = 0;                      // sweeps since the last reset (parity of the halo buffers)
     unsigned long long halo_timeout_ns = 20ull * 1000000000ull;  // CXB_GRID_HALO_TIMEOUT_MS overrides (tests)
-    // m2v planes: a sweep stores only their first and last rows unless eager_m2v (CXB_GRID_EAGER_M2V=1); m2v_pending = the
-    // other rows of the last sweep are not yet rebuilt (flush_m2v)
-    bool eager_m2v = false, m2v_pending = false;
+    // m2v planes and marginals: a sweep stores only their first and last rows unless eager_m2v (CXB_GRID_EAGER_M2V=1), or,
+    // for the marginals, the sweep is the last of an infer_host job; m2v_pending / marg_pending = the other rows of the last
+    // sweep are not yet rebuilt (flush). pend_unary / pend_marg: the evidence that sweep read and the marginal buffer it
+    // wrote, which infer_host may since have switched away from
+    bool eager_m2v = false, m2v_pending = false, marg_pending = false;
+    const unsigned char* pend_unary = nullptr;
+    unsigned char* pend_marg = nullptr;
+    cudaEvent_t ev_fl = nullptr;  // infer_host: the evidence upload waits for a marginal rebuild that reads its buffer
     // after a stream sync: did a halo wait give up on a neighbour?
     int32_t check_halo() {
         if (!peer_halo[0] && !peer_halo[1]) return CXB_OK;
@@ -327,6 +347,7 @@ struct Grid {
             if (q) cudaIpcCloseMemHandle(q);
         if (ev0) cudaEventDestroy(ev0);
         if (ev1) cudaEventDestroy(ev1);
+        if (ev_fl) cudaEventDestroy(ev_fl);
         for (int i = 0; i < 2; ++i) {
             if (ev_in[i]) cudaEventDestroy(ev_in[i]);
             if (ev_sw[i]) cudaEventDestroy(ev_sw[i]);
@@ -373,7 +394,7 @@ struct Grid {
     }
     int32_t reset() {
         CXB_CUDA(cudaSetDevice(device));
-        if (int32_t st = flush_m2v()) return st;  // before the fill below overwrites the m2f planes it reads
+        if (int32_t st = flush(true, true)) return st;  // before the fill below overwrites the m2f planes it reads
         size_t n = (size_t)4 * H * W * K, nh = (size_t)4 * W * K;
         double u = 1.0 / K;
         for (int b = 0; b < 2; ++b) dtype == CXB_F32 ? fill<float>(m2f[b].p, n, u) : fill<double>(m2f[b].p, n, u);
@@ -397,7 +418,7 @@ struct Grid {
         g.W = W;
         g.has_up = has_up;
         g.has_down = has_down;
-        g.eager_m2v = eager_m2v;
+        g.inner_m2v = g.inner_marg = eager_m2v;
         for (int d = 0; d < 4; ++d) {
             g.m2f_cur[d] = m2f[in].p + (size_t)d * plane();
             g.m2f_nxt[d] = m2f[in ^ 1].p + (size_t)d * plane();
@@ -429,7 +450,8 @@ struct Grid {
         }
         return CXB_OK;
     }
-    int32_t sweep(int64_t* n_updates) {
+    // all_marg: store every marginal whatever the mode (the last sweep of an infer_host job)
+    int32_t sweep(int64_t* n_updates, bool all_marg = false) {
         if (!have_unary || !have_msgs) {
             err = "set the unary evidence and reset the messages first";
             return CXB_ERR_STATE;
@@ -438,6 +460,7 @@ struct Grid {
         GridView g = view(cur);
         g.unary = cur_unary ? cur_unary : unary.p;
         g.marg = cur_marg ? cur_marg : marg.p;
+        g.inner_marg |= all_marg;
         // halo buffers are double buffered by sweep parity: sweep s reads parity s & 1 (written by the neighbours' sweep
         // s - 1, or by the caller's exchange) and pushes its own boundary rows into the neighbours' parity (s + 1) & 1
         const size_t par = (size_t)(sweep_no & 1) * 2 * row(), nxt_par = (size_t)((sweep_no + 1) & 1) * 2 * row();
@@ -453,7 +476,10 @@ struct Grid {
         int32_t st = dtype == CXB_F32 ? launch_k<float, 4>(g, false) : launch_k<double, 2>(g, false);
         if (st) return st;
         CXB_CUDA(cudaEventRecord(ev1, stream));
-        m2v_pending = !eager_m2v;
+        m2v_pending = !g.inner_m2v;
+        marg_pending = !g.inner_marg;
+        pend_unary = (const unsigned char*)g.unary;
+        pend_marg = (unsigned char*)g.marg;
         if (fused)  // tell the neighbours: my sweep sweep_no is complete (I am their lower / upper neighbour)
             CXB_LAUNCH(k_halo_signal, 1, 1, 0, stream, peer_flags[0] ? peer_flags[0] + 1 : nullptr, peer_flags[1] ? peer_flags[1] + 0 : nullptr,
                        sweep_no + 1);
@@ -469,18 +495,26 @@ struct Grid {
         }
         return CXB_OK;
     }
-    // rebuild the m2v rows the last sweep did not store, from the m2f planes it read (m2f[cur ^ 1] once it has run); enqueued
-    // on `stream` after the sweep and outside ev0 / ev1
-    int32_t flush_m2v() {
-        if (!m2v_pending) return CXB_OK;
+    // rebuild the m2v rows (m2v) and / or the marginal rows (marg) the last sweep did not store, from the m2f planes it read
+    // (m2f[cur ^ 1] once it has run) and the evidence it read, in one k_potts_m2v launch; enqueued on `stream` after the sweep
+    // and outside ev0 / ev1
+    int32_t flush(bool m2v, bool marg) {
+        m2v = m2v && m2v_pending;
+        marg = marg && marg_pending;
+        if (!m2v && !marg) return CXB_OK;
         CXB_CUDA(cudaSetDevice(device));
         if (H > 2) {
-            const GridView g = view(cur ^ 1);
+            GridView g = view(cur ^ 1);
+            g.inner_m2v = m2v;
+            g.inner_marg = marg;
+            g.unary = pend_unary;
+            g.marg = pend_marg;
             int32_t st = dtype == CXB_F32 ? launch_k<float, 4>(g, true) : launch_k<double, 2>(g, true);
             if (st) return st;
             CXB_CUDA(cudaGetLastError());
         }
-        m2v_pending = false;
+        if (m2v) m2v_pending = false;
+        if (marg) marg_pending = false;
         return CXB_OK;
     }
     // Host entry point of one JOB: evidence from (pinned) host memory, n_sweeps synchronous sweeps, marginals back to host
@@ -494,11 +528,15 @@ struct Grid {
             return CXB_ERR_STATE;
         }
         CXB_CUDA(cudaSetDevice(device));
+        // marginals a plain sweep() left pending are rebuilt now: their evidence buffer may be the one this job uploads into
+        const bool flushed = marg_pending;
+        if (int32_t st = flush(false, true)) return st;
         if (!s_in) {
             CXB_CUDA(unary_alt.reserve(plane()));
             CXB_CUDA(marg_alt.reserve(plane()));
             CXB_CUDA(cudaStreamCreateWithFlags(&s_in, cudaStreamNonBlocking));
             CXB_CUDA(cudaStreamCreateWithFlags(&s_out, cudaStreamNonBlocking));
+            CXB_CUDA(cudaEventCreateWithFlags(&ev_fl, cudaEventDisableTiming));
             for (int i = 0; i < 2; ++i) {
                 CXB_CUDA(cudaEventCreateWithFlags(&ev_in[i], cudaEventDisableTiming));
                 CXB_CUDA(cudaEventCreateWithFlags(&ev_sw[i], cudaEventDisableTiming));
@@ -509,6 +547,10 @@ struct Grid {
         const int b = (int)(job_no & 1);
         unsigned char* U = b ? unary_alt.p : unary.p;
         unsigned char* M = b ? marg_alt.p : marg.p;
+        if (flushed) {
+            CXB_CUDA(cudaEventRecord(ev_fl, stream));
+            CXB_CUDA(cudaStreamWaitEvent(s_in, ev_fl, 0));
+        }
         if (job_no >= 2) CXB_CUDA(cudaStreamWaitEvent(s_in, ev_sw[b], 0));  // the sweeps of job j - 2 have read this evidence buffer
         CXB_CUDA(cudaMemcpyAsync(U, unary_host, plane(), cudaMemcpyHostToDevice, s_in));
         CXB_CUDA(cudaEventRecord(ev_in[b], s_in));
@@ -518,8 +560,8 @@ struct Grid {
         cur_marg = M;
         have_unary = true;
         int64_t upd = 0;
-        for (int k = 0; k < n_sweeps; ++k) {
-            int32_t st = sweep(&upd);
+        for (int k = 0; k < n_sweeps; ++k) {  // the last sweep stores every marginal: the download below needs no rebuild
+            int32_t st = sweep(&upd, k + 1 == n_sweeps);
             if (st) return st;
         }
         CXB_CUDA(cudaEventRecord(ev_sw[b], stream));
@@ -586,6 +628,7 @@ const char* cxb_grid_last_error(cxb_grid* g) { return g ? GR(g)->err.c_str() : "
 int32_t cxb_grid_set_unary(cxb_grid* g, const void* unary_host) try {
     Grid* h = GR(g);
     GR_CUDA(g, cudaSetDevice(h->device));
+    if (int32_t st = h->flush(false, true)) return st;  // the pending marginals are those of the evidence about to be replaced
     GR_CUDA(g, cudaMemcpyAsync(h->cur_unary ? h->cur_unary : h->unary.p, unary_host, h->plane(), cudaMemcpyHostToDevice, h->stream));
     GR_CUDA(g, cudaStreamSynchronize(h->stream));
     h->have_unary = true;
@@ -660,6 +703,7 @@ int64_t cxb_grid_halo_elems(cxb_grid* g) try { return GR(g)->W * GR(g)->K; } CXB
 int32_t cxb_grid_get_marginals(cxb_grid* g, void* out_host) try {
     Grid* h = GR(g);
     GR_CUDA(g, cudaSetDevice(h->device));
+    if (int32_t st = h->flush(false, true)) return st;
     GR_CUDA(g, cudaMemcpyAsync(out_host, h->cur_marg ? h->cur_marg : h->marg.p, h->plane(), cudaMemcpyDeviceToHost, h->stream));
     GR_CUDA(g, cudaStreamSynchronize(h->stream));
     return h->check_halo();
@@ -674,7 +718,7 @@ int32_t cxb_grid_get_messages(cxb_grid* g, int32_t which, void* out_host) try {
     const unsigned char* src = which < 4 ? h->m2v.p + (size_t)which * h->plane() : h->m2f[h->cur].p + (size_t)(which - 4) * h->plane();
     GR_CUDA(g, cudaSetDevice(h->device));
     if (which < 4)
-        if (int32_t st = h->flush_m2v()) return st;
+        if (int32_t st = h->flush(true, false)) return st;
     GR_CUDA(g, cudaMemcpyAsync(out_host, src, h->plane(), cudaMemcpyDeviceToHost, h->stream));
     GR_CUDA(g, cudaStreamSynchronize(h->stream));
     return CXB_OK;

@@ -340,7 +340,8 @@ int32_t cxb_grid_create(int32_t device, int32_t dtype, int64_t rows, int64_t col
                         int32_t has_upper_neighbour, int32_t has_lower_neighbour, cxb_grid** out);
 void cxb_grid_destroy(cxb_grid* g);
 const char* cxb_grid_last_error(cxb_grid* g);
-/* set_value!(m2v(v, unary_v), u_v): host [rows][cols][K] engine dtype */
+/* set_value!(m2v(v, unary_v), u_v): host [rows][cols][K] engine dtype. Marginals of the last sweep that are not yet
+ * rebuilt (cxb_grid_get_marginals) are rebuilt from the old evidence first, so they stay those of the evidence it read. */
 int32_t cxb_grid_set_unary(cxb_grid* g, const void* unary_host);
 /* set every pairwise m2f to the uniform initial message (protocol B step 1) */
 int32_t cxb_grid_reset_messages(cxb_grid* g);
@@ -360,7 +361,10 @@ int64_t cxb_grid_halo_elems(cxb_grid* g);
 int32_t cxb_grid_p2p_export(cxb_grid* g, void* handles_out);
 int32_t cxb_grid_p2p_connect_ipc(cxb_grid* g, int32_t direction, const void* neighbour_handles);
 int32_t cxb_grid_p2p_connect_local(cxb_grid* g, int32_t direction, cxb_grid* neighbour);
-/* marginals [rows][cols][K] engine dtype, D2H */
+/* marginals [rows][cols][K] engine dtype, D2H. A sweep computes every marginal but stores only those of its first and last
+ * rows (every row in the last sweep of a cxb_grid_infer_host job); the first call after a sweep rebuilds the others, bit
+ * for bit, from the m2f messages and the evidence that sweep read (one extra kernel on the grid's stream, about 26 GB of
+ * traffic at 8192^2, K = 16 fp32; a second call launches nothing). Before any sweep it returns zeros. */
 int32_t cxb_grid_get_marginals(cxb_grid* g, void* out_host);
 /* One JOB through host buffers (the e2e path of config 4): unary evidence [rows][cols][K] from (pinned) host memory, n_sweeps
  * synchronous sweeps, marginals back to (pinned) host memory. Asynchronous and pipelined over three streams: the call returns
@@ -371,8 +375,9 @@ int32_t cxb_grid_infer_host(cxb_grid* g, const void* unary_host, void* marginals
 /* message planes for parity: which = 0..3 m2v from the (up,left,right,down) factor, 4..7 m2f to them; D2H.
  * A sweep computes every m2v but stores only those of its first and last rows; the first read of an m2v plane after a
  * sweep rebuilds the other rows, bit for bit, from the m2f messages that sweep read (one extra kernel on the grid's stream,
- * about 34 GB of traffic at 8192^2, K = 16 fp32; later reads of the same sweep's planes launch nothing).
- * CXB_GRID_EAGER_M2V=1 at cxb_grid_create stores every m2v every sweep instead. */
+ * about 34 GB of traffic at 8192^2, K = 16 fp32; later reads of the same sweep's planes launch nothing). Reading 4..7
+ * rebuilds nothing, and reading 0..3 leaves pending marginals to cxb_grid_get_marginals.
+ * CXB_GRID_EAGER_M2V=1 at cxb_grid_create stores every m2v and every marginal every sweep instead. */
 int32_t cxb_grid_get_messages(cxb_grid* g, int32_t which, void* out_host);
 void* cxb_grid_stream(cxb_grid* g);
 int32_t cxb_grid_last_kernel_ms(cxb_grid* g, float* ms_out);

@@ -1,6 +1,7 @@
 // stream_mix.cu — streaming bandwidth of a B200 by read : write mix. The Gaussian chain kernel (config 2) reads 12 B and
 // writes 52 B per state variable (forward recursion 4 : 24, backward 12 : 24 ... 8 : 28), the copy that defines the roofline
-// peak is 1 : 1. Build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o stream_mix stream_mix.cu
+// peak is 1 : 1; the Potts sweep (config 4) reads 5 and writes 4 16-byte vectors per lane.
+// Build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o stream_mix stream_mix.cu
 #include <cstdio>
 #include <cstdlib>
 #include <cstdint>
@@ -38,8 +39,8 @@ __global__ void k16(const float4* __restrict__ src, float4* __restrict__ dst, si
 int main() {
     const size_t n = (size_t)64 << 20;  // 64 Mi elements of 8 bytes = 512 MiB per plane (the chain planes: 65,536 x 1,024 x 8 B)
     float2 *src, *dst;
-    CK(cudaMalloc(&src, n * 8 * 4)); CK(cudaMalloc(&dst, n * 8 * 7));
-    CK(cudaMemset(src, 0, n * 8 * 4)); CK(cudaMemset(dst, 0, n * 8 * 7));
+    CK(cudaMalloc(&src, n * 8 * 5)); CK(cudaMalloc(&dst, n * 8 * 7));
+    CK(cudaMemset(src, 0, n * 8 * 5)); CK(cudaMemset(dst, 0, n * 8 * 7));
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     auto run = [&](const char* name, auto launch, double bytes) {
         for (int i = 0; i < 2; ++i) launch();
@@ -68,5 +69,6 @@ int main() {
     run("16-byte elements, read 1 : write 4", [&] { k16<1, 4><<<grid, blk>>>(s16, d16, n16); }, n16 * 16.0 * 5);
     run("16-byte elements, read 2 : write 3", [&] { k16<2, 3><<<grid, blk>>>(s16, d16, n16); }, n16 * 16.0 * 5);
     run("16-byte elements, read 1 : write 6", [&] { k16<1, 6><<<grid, blk>>>(s16, d16, n16); }, n16 * 16.0 * 7);
+    run("16-byte elements, read 5 : write 4 (Potts sweep)", [&] { k16<5, 4><<<grid, blk>>>(s16, d16, n16); }, n16 * 16.0 * 9);
     return 0;
 }

@@ -1,8 +1,9 @@
-"""A/B of the Potts sweep at the benchmarked size (8192^2, K = 16, fp32): every m2v plane stored each sweep
-(CXB_GRID_EAGER_M2V=1) against the default, where a sweep stores the m2v of its first and last rows only and the first read
-of an m2v plane rebuilds the others (k_potts_m2v). The two grids take 60 GB each, so they are created one after the other,
-alternating, for `rounds` rounds. Per arm: 3 x 50 warm-up sweeps, 50 sweeps timed with CUDA events on the library's stream,
-then last_kernel_ms over 10 sweeps; the lazy arm also times one rebuild with torch.profiler.
+"""A/B of the Potts sweep at the benchmarked size (8192^2, K = 16, fp32): every m2v plane and every marginal stored each
+sweep (CXB_GRID_EAGER_M2V=1) against the default, where a sweep stores the m2v and the marginals of its first and last rows
+only and the first read of an m2v plane or of the marginals rebuilds the others (k_potts_m2v). The two grids take 60 GB
+each, so they are created one after the other, alternating, for `rounds` rounds. Per arm: 3 x 50 warm-up sweeps, 50 sweeps
+timed with CUDA events on the library's stream, then last_kernel_ms over 10 sweeps; the lazy arm also times the two rebuilds
+(marginals, then m2v planes) with torch.profiler.
 Usage: python profiles/time_potts_m2v.py [N] [rounds]"""
 import gc
 import os
@@ -32,14 +33,16 @@ for i in range(0, N, 256):
 pix = N * N
 m2v = 2 * (N - 1) * N * 2
 bytes_all = 64 * ((m2v + pix) + (2 * m2v + pix))  # 896 B per interior pixel: reads 4 m2f + unary, writes 4 m2v + 4 m2f + marginal
-bytes_lazy = 64 * ((m2v + pix) + (m2v + pix))  # 640 B per interior pixel: without the m2v stores
+bytes_lazy = 64 * ((m2v + pix) + m2v)  # 576 B per interior pixel: without the m2v and marginal stores
+bytes_rb_marg = 64 * ((m2v + pix) + pix)  # marginal rebuild: reads 4 m2f + unary, writes the marginal
+bytes_rb_m2v = 64 * 2 * m2v  # m2v rebuild: reads 4 m2f, writes 4 m2v
 
 
-def rebuild_ms(g):
-    """device time of the k_potts_m2v launch that the first m2v read after a sweep enqueues"""
+def rebuild_ms(g, read):
+    """device time of the k_potts_m2v launch that read(g), the first read after a sweep, enqueues"""
     try:
         with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-            g.get_messages(0)
+            read(g)
         us = [e.time_range.elapsed_us() for e in prof.events() if "k_potts_m2v" in e.name]
         return us[0] / 1e3 if us else None
     except Exception as ex:  # noqa: BLE001 - the A/B numbers do not depend on it
@@ -67,7 +70,7 @@ def arm(eager):
     for _ in range(10):
         g.sweep()
         kms.append(g.last_kernel_ms())
-    rb = None if eager else rebuild_ms(g)
+    rb = None if eager else (rebuild_ms(g, lambda x: x.get_marginals()), rebuild_ms(g, lambda x: x.get_messages(0)))
     del g
     gc.collect()
     return ms, statistics.mean(kms), rb
@@ -78,10 +81,13 @@ for r in range(ROUNDS):
     for eager in (True, False):
         ms, kms, rb = arm(eager)
         res[eager].append((ms, kms))
-        name = "eager (every m2v stored)" if eager else "lazy (m2v rebuilt on read)"
-        extra = f", rebuild of the m2v planes {rb:.3f} ms = {(64 * 2 * m2v) / (rb * 1e6):.0f} GB/s" if rb else ""
-        print(f"round {r} {name:28s}: {ms:.3f} ms per sweep (events, {SWEEPS} sweeps), last_kernel_ms {kms:.3f}{extra}", flush=True)
-print(f"{N}^2, K = {K}: bytes per sweep {bytes_all / 1e9:.2f} GB (896 B per pixel) / {bytes_lazy / 1e9:.2f} GB (640 B per pixel)")
+        name = "eager (every value stored)" if eager else "lazy (rebuilt on read)"
+        extra = ""
+        for what, t, nb in zip(("marginals", "m2v planes"), rb or (), (bytes_rb_marg, bytes_rb_m2v)):
+            if t:
+                extra += f", rebuild of the {what} {t:.3f} ms = {nb / (t * 1e6):.0f} GB/s"
+        print(f"round {r} {name:26s}: {ms:.3f} ms per sweep (events, {SWEEPS} sweeps), last_kernel_ms {kms:.3f}{extra}", flush=True)
+print(f"{N}^2, K = {K}: bytes per sweep {bytes_all / 1e9:.2f} GB (896 B per pixel) / {bytes_lazy / 1e9:.2f} GB (576 B per pixel)")
 for eager in (True, False):
     ev = [m for m, _ in res[eager]]
     kk = [k for _, k in res[eager]]
@@ -89,6 +95,6 @@ for eager in (True, False):
     print(f"{'eager' if eager else 'lazy':5s}: {mean:.3f} ms per sweep (events), spread {min(ev):.3f} .. {max(ev):.3f} "
           f"({(max(ev) - min(ev)) / mean * 100:.2f} %); last_kernel_ms {statistics.mean(kk):.3f} "
           f"({min(kk):.3f} .. {max(kk):.3f}); {bytes_all / (mean * 1e6):.0f} GB/s on the 896-B count, "
-          f"{bytes_lazy / (mean * 1e6):.0f} GB/s on the 640-B count")
+          f"{bytes_lazy / (mean * 1e6):.0f} GB/s on the 576-B count")
 ratio = [a[0] / b[0] for a, b in zip(res[True], res[False])]
 print(f"eager / lazy per sweep: {statistics.mean(ratio):.3f} (rounds: {', '.join(f'{x:.3f}' for x in ratio)})")
