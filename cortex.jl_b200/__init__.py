@@ -21,6 +21,6 @@ from .inference_engine import *  # noqa: F401,F403
 from .inference_engine import _as_ids  # noqa: F401
 from .structured import GaussianChainBatch, HmmBatch, PairwiseGraph, PottsGrid  # noqa: F401
 from .debug import signal_to_dot  # noqa: F401
-from .sharding import HaloExchanger, batch_shard, connect_row_neighbours, device_tensor, row_shard  # noqa: F401
+from .sharding import HaloExchanger, batch_shard, connect_row_neighbours, device_tensor, row_shard, shard_couplings  # noqa: F401
 
 __version__ = "0.1.0"

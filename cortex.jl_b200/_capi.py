@@ -110,6 +110,7 @@ _STRUCTURED = {
     "grid_destroy": (None, [vp]),
     "grid_last_error": (C.c_char_p, [vp]),
     "grid_set_unary": (i32, [vp, vp]),
+    "grid_set_couplings": (i32, [vp, f64p, f64p]),
     "grid_reset_messages": (i32, [vp]),
     "grid_sweep": (i32, [vp, i64p]),
     "grid_halo_send_ptr": (vp, [vp, i32]),

@@ -24,6 +24,12 @@
 // `nxt`), every value is read exactly once.  Row sharding: the up/down messages of the first/last local row
 // are contiguous rows of the `up`/`down` planes and are exchanged with the neighbour ranks between sweeps
 // (halo_send_ptr / halo_recv_ptr), see cortex.jl_b200/grid.py.
+//
+// Per-edge couplings (cxb_grid_set_couplings): factor e has its own beta_e; the closed form above holds per factor with
+// w_e = e^beta_e - 1, converted on the host exactly as the uniform w is, so equal couplings give the uniform grid bit for
+// bit. The kernels' PE instantiations load w_e from two planes in the engine dtype, w_h [H][W] and w_v [H + 1][W] (rows 0
+// and H: the cut edges), +8 B per pixel at fp32; the PE = false instantiations are the uniform kernels unchanged. The lazy
+// rebuilds read the same planes, so set_couplings first flushes whatever the last sweep left pending.
 #include <cmath>
 
 #include <cstring>
@@ -146,8 +152,24 @@ struct GridView {
     void* peer_down;        // lower neighbour's halo_up slot: receives the last row of plane `down`
 };
 
-template <class T, int K, int E>
-__global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
+// Per-edge couplings (cxb_grid_set_couplings), w = e^beta - 1 of each of a pixel's four factors, from the planes wh[H][W]
+// (factor to the right of pixel (i, j); last column unused) and wv[H + 1][W] (factor above local row i; rows 0 and H are the
+// cut edges); pix = i * W + j. An absent factor's coupling is never used; the left one is not even loaded, as pix - 1 is
+// outside the plane at pixel 0. Each weight is loaded by both of its pixels, the second load hits L1 or L2.
+template <class T>
+__device__ __forceinline__ void couplings(const T* __restrict__ wh, const T* __restrict__ wv, long long W, long long pix, bool has_left,
+                                          T w, T (&wd)[4]) {
+    wd[0] = __ldg(wv + pix);
+    wd[1] = has_left ? __ldg(wh + pix - 1) : w;
+    wd[2] = __ldg(wh + pix);
+    wd[3] = __ldg(wv + pix + W);
+}
+
+// PE: every factor has its own coupling (couplings()); otherwise all have `w`, and wh / wv are unused. They follow `w`, and
+// PE = false passes `w` itself to potts_m2v, so the uniform kernels compile to the instruction stream they had before
+// per-edge couplings existed.
+template <class T, int K, int E, bool PE>
+__global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w, const T* __restrict__ wh, const T* __restrict__ wv) {
     constexpr int LP = K / E;  // lanes per pixel
     static_assert(LP >= 1 && LP <= 32 && (LP & (LP - 1)) == 0, "K / E must be a power of two <= 32");
     const long long npix = g.H * g.W;
@@ -190,10 +212,12 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
     // loop phase
     // rows 0 and H - 1 (every row when H <= 2) in one unsigned compare; i == 0 || i + 1 == g.H costs the fp32 sweep registers
     const bool edge_row = (unsigned long long)(pix - g.W) >= (unsigned long long)(npix - 2 * g.W);
+    T wd[4];
+    if constexpr (PE) couplings<T>(wh, wv, g.W, pix, ex[1], w, wd);
     T mv[4][E];
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
-        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], valid && (g.inner_m2v || edge_row), g.m2v[d], o);
+        potts_m2v<T, E, LP>(in[d], ex[d], PE ? wd[d] : w, mv[d], valid && (g.inner_m2v || edge_row), g.m2v[d], o);
     }
     // final phase: the linked m2f, then the marginal (products in ascending factor order, left to right; the marginal last
     // keeps the fp32 sweep at 48 registers)
@@ -225,8 +249,8 @@ __global__ void __launch_bounds__(256) k_potts_sweep(GridView g, T w) {
 // (g.unary): both stay intact until the next sweep, whose own values supersede these, or until the host flushes (reset,
 // set_unary, infer_host). Rows 1 .. H - 2 take their up and down inputs from this shard's planes, never from a halo buffer.
 // Lane layout as in k_potts_sweep; no m2v store where the factor is absent, so those slots keep the zeros of init.
-template <class T, int K, int E>
-__global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
+template <class T, int K, int E, bool PE>
+__global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w, const T* __restrict__ wh, const T* __restrict__ wv) {
     constexpr int LP = K / E;
     const long long npix = (g.H - 2) * g.W;
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -254,10 +278,12 @@ __global__ void __launch_bounds__(256) k_potts_m2v(GridView g, T w) {
         }
     }
     if (g.inner_marg) load_vec<T, E>((const T*)g.unary + o, un);
+    T wd[4];
+    if constexpr (PE) couplings<T>(wh, wv, g.W, pix, ex[1], w, wd);
     T mv[4][E];
 #pragma unroll
     for (int d = 0; d < 4; ++d) {
-        potts_m2v<T, E, LP>(in[d], ex[d], w, mv[d], valid && g.inner_m2v, g.m2v[d], o);
+        potts_m2v<T, E, LP>(in[d], ex[d], PE ? wd[d] : w, mv[d], valid && g.inner_m2v, g.m2v[d], o);
     }
     if (g.inner_marg) potts_marginal<T, E, LP>(un, mv, ex, valid, g.marg, o);
 }
@@ -325,6 +351,10 @@ struct Grid {
     const unsigned char* pend_unary = nullptr;
     unsigned char* pend_marg = nullptr;
     cudaEvent_t ev_fl = nullptr;  // infer_host: the evidence upload waits for a marginal rebuild that reads its buffer
+    // per-edge couplings (cxb_grid_set_couplings), w = e^beta - 1 in the engine dtype: w_h [H][W], w_v [H + 1][W]; reserved on
+    // first use. coupled = the kernels read them instead of the create-time beta
+    DBuf<unsigned char> w_h, w_v;
+    bool coupled = false;
     // after a stream sync: did a halo wait give up on a neighbour?
     int32_t check_halo() {
         if (!peer_halo[0] && !peer_halo[1]) return CXB_OK;
@@ -430,15 +460,22 @@ struct Grid {
     template <class T, int E>
     int32_t launch_k(const GridView& g, bool m2v_only) {
         const T w = (T)(std::exp(beta) - 1.0);
+        const T* wh = coupled ? (const T*)w_h.p : nullptr;
+        const T* wv = coupled ? (const T*)w_v.p : nullptr;
         long long threads = (m2v_only ? H - 2 : H) * W * (K / E);
         unsigned grid = cdiv((size_t)threads, 256);
         switch (K / E) {
+#define LAUNCH(KERNEL, LPV, PE) CXB_LAUNCH((KERNEL<T, LPV * E, E, PE>), grid, 256, 0, stream, g, w, wh, wv)
 #define CASE(LPV)                                                                                      \
     case LPV:                                                                                          \
-        if (m2v_only)                                                                                  \
-            CXB_LAUNCH((k_potts_m2v<T, LPV * E, E>), grid, 256, 0, stream, g, w);                      \
+        if (m2v_only && coupled)                                                                       \
+            LAUNCH(k_potts_m2v, LPV, true);                                                            \
+        else if (m2v_only)                                                                             \
+            LAUNCH(k_potts_m2v, LPV, false);                                                           \
+        else if (coupled)                                                                              \
+            LAUNCH(k_potts_sweep, LPV, true);                                                          \
         else                                                                                           \
-            CXB_LAUNCH((k_potts_sweep<T, LPV * E, E>), grid, 256, 0, stream, g, w);                    \
+            LAUNCH(k_potts_sweep, LPV, false);                                                         \
         break;
             CASE(1)
             CASE(2)
@@ -447,7 +484,48 @@ struct Grid {
             CASE(16)
             CASE(32)
 #undef CASE
+#undef LAUNCH
         }
+        return CXB_OK;
+    }
+    // cxb_grid_set_couplings: every value is checked before any device state changes; both null = back to the uniform beta
+    template <class T>
+    int32_t set_couplings(const double* hz, const double* vt) {
+        if (!hz != !vt) {
+            err = "set_couplings: give both coupling arrays, or neither (back to the uniform beta)";
+            return CXB_ERR_BAD_ARG;
+        }
+        std::vector<T> h, v;
+        if (hz) {
+            h.assign((size_t)H * W, T(0));
+            v.assign((size_t)(H + 1) * W, T(0));
+            auto conv = [&](double beta, T& out) {
+                const T w = (T)(std::exp(beta) - 1.0);  // the expression of launch_k: equal couplings give the uniform grid
+                if (!std::isfinite(beta) || !std::isfinite(w)) {
+                    err = "set_couplings: beta " + std::to_string(beta) + " is not finite, or exp(beta) - 1 overflows the engine dtype";
+                    return false;
+                }
+                out = w;
+                return true;
+            };
+            for (long long i = 0; i < H; ++i)
+                for (long long j = 0; j + 1 < W; ++j)
+                    if (!conv(hz[i * (W - 1) + j], h[i * W + j])) return CXB_ERR_BAD_ARG;
+            for (long long i = has_up ? 0 : 1; i <= (has_down ? H : H - 1); ++i)  // rows 0 and H only with a neighbour
+                for (long long j = 0; j < W; ++j)
+                    if (!conv(vt[i * W + j], v[i * W + j])) return CXB_ERR_BAD_ARG;
+        }
+        CXB_CUDA(cudaSetDevice(device));
+        // the pending m2v / marginal rows of the last sweep are rebuilt with the couplings it read
+        if (int32_t st = flush(true, true)) return st;
+        if (hz) {
+            CXB_CUDA(w_h.reserve(h.size() * sizeof(T)));
+            CXB_CUDA(w_v.reserve(v.size() * sizeof(T)));
+            CXB_CUDA(cudaMemcpyAsync(w_h.p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, stream));
+            CXB_CUDA(cudaMemcpyAsync(w_v.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, stream));
+        }
+        CXB_CUDA(cudaStreamSynchronize(stream));
+        coupled = hz != nullptr;
         return CXB_OK;
     }
     // all_marg: store every marginal whatever the mode (the last sweep of an infer_host job)
@@ -633,6 +711,10 @@ int32_t cxb_grid_set_unary(cxb_grid* g, const void* unary_host) try {
     GR_CUDA(g, cudaStreamSynchronize(h->stream));
     h->have_unary = true;
     return CXB_OK;
+} CXB_ABI_CATCH(CXB_ERR_INTERNAL)
+int32_t cxb_grid_set_couplings(cxb_grid* g, const double* horizontal, const double* vertical) try {
+    Grid* h = GR(g);
+    return h->dtype == CXB_F32 ? h->set_couplings<float>(horizontal, vertical) : h->set_couplings<double>(horizontal, vertical);
 } CXB_ABI_CATCH(CXB_ERR_INTERNAL)
 int32_t cxb_grid_reset_messages(cxb_grid* g) try { return GR(g)->reset(); } CXB_ABI_CATCH(CXB_ERR_INTERNAL)
 int32_t cxb_grid_sweep(cxb_grid* g, int64_t* n_updates_out) try { return GR(g)->sweep(n_updates_out); } CXB_ABI_CATCH(CXB_ERR_INTERNAL)

@@ -26,6 +26,28 @@ def row_shard(n_rows: int, world: int, rank: int) -> Tuple[int, int, bool, bool]
     return row0, rows, rank > 0, rank < world - 1
 
 
+def shard_couplings(horizontal, vertical, row0: int, rows: int):
+    """This row block's arguments of `PottsGrid.set_couplings`, from the global per-edge couplings of an H x W grid:
+    `horizontal[H][W-1]` (between (i, j) and (i, j+1)) and `vertical[H-1][W]` (between rows i and i+1). Returns
+    (horizontal[rows][W-1], vertical[rows+1][W]): local row r of the vertical array is the factor between global rows
+    row0 + r - 1 and row0 + r, so rows 0 and `rows` are the cut edges, zeros where there is no neighbour. Two neighbours
+    cut their shared edge from the same global row, so they agree on it."""
+    import numpy as np
+
+    hz = np.asarray(horizontal, dtype=np.float64)
+    vt = np.asarray(vertical, dtype=np.float64)
+    H = hz.shape[0]
+    W = vt.shape[1] if vt.ndim == 2 else hz.shape[1] + 1
+    if hz.shape != (H, W - 1) or vt.shape != (H - 1, W):
+        raise ValueError(f"global couplings must be horizontal [H][W-1] and vertical [H-1][W], got {hz.shape} and {vt.shape}")
+    if not (0 <= row0 and rows > 0 and row0 + rows <= H):
+        raise ValueError(f"rows [{row0}, {row0 + rows}) are not inside a grid of {H} rows")
+    v = np.zeros((rows + 1, W))
+    lo, hi = max(row0, 1), min(row0 + rows, H - 1)  # local row r <-> global edge row row0 + r - 1, which exists for 1..H-1
+    v[lo - row0:hi - row0 + 1] = vt[lo - 1:hi]
+    return np.ascontiguousarray(hz[row0:row0 + rows]), v
+
+
 class HaloExchanger:
     """Per-sweep halo exchange between row-neighbour ranks. `dist` is torch.distributed (any backend)."""
 

@@ -127,6 +127,22 @@ class PottsGrid(_Handle):
         assert u.shape == (self.H, self.W, self.K)
         self.check(self.api.grid_set_unary(self.h, u.ctypes.data))
 
+    def set_couplings(self, horizontal, vertical):
+        """Per-edge coupling strengths, psi_e[a][b] = exp(beta_e [a==b]) (``cxb_grid_set_couplings``): ``horizontal[rows][cols-1]``
+        between (i, j) and (i, j+1); ``vertical[rows+1][cols]`` between local rows i-1 and i, row 0 and row ``rows`` being the cut
+        edges to the shards above and below (``sharding.shard_couplings`` cuts them from global arrays). ``None, None``
+        returns to the create-time beta. Sweeps already enqueued keep the couplings they were enqueued with."""
+        if horizontal is None and vertical is None:
+            self.check(self.api.grid_set_couplings(self.h, None, None))
+            return
+        hz = np.ascontiguousarray(horizontal, dtype=np.float64)
+        vt = np.ascontiguousarray(vertical, dtype=np.float64)
+        if hz.shape != (self.H, self.W - 1) or vt.shape != (self.H + 1, self.W):
+            raise ValueError(f"couplings of a {self.H} x {self.W} shard are horizontal [{self.H}][{self.W - 1}] and vertical "
+                             f"[{self.H + 1}][{self.W}], got {hz.shape} and {vt.shape}")
+        hz = hz if hz.size else np.zeros(1)  # a one-column shard has no horizontal factor; the library still wants a pointer
+        self.check(self.api.grid_set_couplings(self.h, hz.ctypes.data_as(capi.f64p), vt.ctypes.data_as(capi.f64p)))
+
     def reset_messages(self):
         self.check(self.api.grid_reset_messages(self.h))
 

@@ -343,6 +343,16 @@ const char* cxb_grid_last_error(cxb_grid* g);
 /* set_value!(m2v(v, unary_v), u_v): host [rows][cols][K] engine dtype. Marginals of the last sweep that are not yet
  * rebuilt (cxb_grid_get_marginals) are rebuilt from the old evidence first, so they stay those of the evidence it read. */
 int32_t cxb_grid_set_unary(cxb_grid* g, const void* unary_host);
+/* Per-edge coupling strengths of this shard's pairwise factors, psi_e[a][b] = exp(beta_e [a==b]); float64 host arrays:
+ *   horizontal[rows][cols-1]  beta of the factor between (i, j) and (i, j+1)
+ *   vertical[rows+1][cols]    beta of the factor between local rows i-1 and i; row 0 = the cut edge to the shard above
+ *                             (read only with has_upper_neighbour), row `rows` = the cut edge below (only with has_lower)
+ * They replace the create-time beta for every pairwise factor until the call is repeated with both pointers NULL (back to
+ * the uniform beta). Stream-ordered: sweeps enqueued before the call read the old couplings. m2v / marginal rows of the
+ * last sweep that are not yet rebuilt are rebuilt first, with the couplings that sweep read. A non-finite beta, or
+ * exp(beta) - 1 not finite in the engine dtype: CXB_ERR_BAD_ARG and nothing changes. Row neighbours must be given the
+ * same beta for their shared cut edge. */
+int32_t cxb_grid_set_couplings(cxb_grid* g, const double* horizontal, const double* vertical);
 /* set every pairwise m2f to the uniform initial message (protocol B step 1) */
 int32_t cxb_grid_reset_messages(cxb_grid* g);
 /* one synchronous sweep on the local rows; halo rows must have been exchanged (cxb_grid_halo_*) */
